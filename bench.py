@@ -2,7 +2,7 @@
 """Benchmark of the track-likelihood hot path (BASELINE.json metric: track-steps/s of one -log L
 evaluation, 2-state 2-D, frame_len = 8, sim_FOV synthetic tracks of length 10-30).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--tracks T] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--tracks T] [--impl ours|reference] [--dump-outputs DIR]
 
 A *step* is one objective evaluation over the resident data set (plan kernels, replay kernels,
 device reduction; plus one 8-byte all-reduce when N > 1).  Plan and replay are launched per group of
@@ -22,6 +22,11 @@ ranks through the API).
 --impl reference times the CPU path instead: the numpy oracle port of the reference algorithm
 (the reference is pure Python and does not travel to the GPU box) on all host cores, on a bounded
 sample of the same workload.
+
+--dump-outputs DIR writes what the timed path returned in its last timed step to DIR/sum_logp.npy (float64, shape
+[1]: the log-likelihood summed over the data set, after the all-reduce when N > 1).  The data set is generated from
+fixed seeds and the parameter table of a step depends only on its index, so two builds run with the same arguments
+can be compared output for output.
 """
 from __future__ import annotations
 
@@ -115,6 +120,14 @@ def cpu_baseline(st):
     if out.returncode != 0:
         raise RuntimeError("cpu_baseline leg failed: " + out.stderr[-2000:])
     return json.loads(out.stdout.strip().splitlines()[-1])
+
+
+def dump_outputs(path, sum_logp):
+    """--dump-outputs: the result of the last timed step as `path`/sum_logp.npy."""
+    import numpy as np
+
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "sum_logp.npy"), np.array([sum_logp], dtype=np.float64))
 
 
 class ClockSampler(threading.Thread):
@@ -468,6 +481,8 @@ def run_reference(args):
     for _ in range(args.steps):
         val = orc.neg_log_likelihood(st, model, workers=cores)
     dt = time.perf_counter() - t
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, -val)
     v = steps_per_eval * args.steps / dt
     sample = f"{n} sim_FOV tracks ({steps_per_eval} track-steps, whole 2000-track chunks) per step, numpy oracle port, fork pool"
     print(json.dumps({
@@ -496,6 +511,8 @@ def main():
     ap.add_argument("--e2e-steps", type=int, default=10)
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-secondary", action="store_true", help="skip the strong / api / secondary blocks (profiling runs)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the result of the last timed step to DIR/sum_logp.npy (rank 0)")
     args = ap.parse_args()
     if args.warmup < 3:
         args.warmup = 3
@@ -580,6 +597,7 @@ def main():
     ev1.record()
     barrier()
     ms = ev0.elapsed_time(ev1)
+    last = float(buf.item()) if args.dump_outputs else None  # result of the last timed step (buf is reused below)
     eng.sum_logp_async(p, buf.data_ptr(), stream)  # (untimed) the base parameters again: `sum_logp` of the line
     if world > 1:
         dist.all_reduce(buf)
@@ -769,6 +787,8 @@ def main():
             "secondary": secondary,
         }
         print(json.dumps(line))
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, last)
     ts.close()
     if world > 1:
         dist.destroy_process_group()

@@ -148,30 +148,24 @@ def test_oracle_vs_live_reference(cfg):
     np.testing.assert_allclose(got, ref, rtol=1e-13)
 
 
-@needs_ref
-def test_oracle_vs_live_reference_tracks_csv_known_answer():
-    """Known-answer values of SURVEY.md §6 on Tutorials/tracks.csv (regenerated, not hard-coded bitwise)."""
-    trk = ref_loader.load_tracking()
-    rd = ref_loader.load_readers()
-    with contextlib.redirect_stdout(io.StringIO()):
-        tracks, _, _ = rd.read_table(os.path.join(ref_loader.REFERENCE_ROOT, "Tutorials", "tracks.csv"), lengths=np.arange(5, 50),
-                                     dist_th=0.3, frames_boundaries=[0, 10000], fmt="csv", colnames=["X", "Y", "frame", "track_ID"],
-                                     opt_colnames=[], remove_no_disp=True)
-    keys = sorted(tracks, key=int)
-    st = [tracks[k] for k in keys if len(tracks[k])]
+@pytest.mark.parametrize("fl,ref", [(4, -16372.353108152653), (6, -16372.631616957766), (8, -16373.513684485983)])
+def test_oracle_matches_reference_known_answers_on_tutorial_tracks(fl, ref):
+    """Known-answer values of SURVEY.md §6: the unmodified reference's cum_Proba_Cs on Tutorials/tracks.csv at fixed
+    parameters.  The tracks are the ones the reference's own reader produced from that file (stored in
+    fit_tracks_csv.npz by tests/golden/make_golden.py:make_fit_case, same reader arguments)."""
+    z = np.load(os.path.join(GOLDEN, "fit_tracks_csv.npz"))
+    st = [z["C" + k] for k in z["keys"]]
     assert sum(len(a) for a in st) == 613
-    from lmfit import Parameters
+    from extrack_b200 import tracking as xt
+    from extrack_b200._lmfit_compat import Parameters
 
     p = Parameters()
     for k, v in dict(D0=1e-5, D1=0.35, LocErr=0.02, F0=0.54, p01=0.077, p10=0.138, pBL=0.11).items():
         p.add(k, value=v)
     p.add("F1", expr="1-F0")
-    LocErr, ds, Fs, TrMat, pBL = trk.extract_params(p, 0.02, 2, 1)
-    model = orc.Model(LocErr[0].reshape(-1), ds, Fs, TrMat, pBL, [1], 1, 6, st[0].shape[1], 0.2, 120)
+    LocErr, ds, Fs, TrMat, pBL = xt.extract_params(p, 0.02, 2, 1)
+    model = orc.Model(LocErr[0].reshape(-1), ds, Fs, TrMat, pBL, [1], 1, fl, st[0].shape[1], 0.2, 120)
     got = orc.neg_log_likelihood(st, model)
-    assert abs(got - (-16372.631616957766)) < 1e-6
-    with contextlib.redirect_stdout(io.StringIO()):
-        ref = trk.cum_Proba_Cs(p, st, 0.02, [1], None, 2, 1, 6, 0, 1, 1, 0.2, 120)
     assert abs(got - ref) / abs(ref) < 1e-13
 
 
