@@ -1,7 +1,8 @@
 """extrack_b200 — B200-native (sm_100a CUDA) track-likelihood engine behind ExTrack's Python API.
 
 Only the hot path of ``extrack.tracking`` is provided: ``param_fitting`` / ``cum_Proba_Cs`` /
-``Proba_Cs`` / ``predict_Bs`` and the parameter builders, plus the data formats either side of it:
+``Proba_Cs`` / ``predict_Bs`` and the parameter builders (plus ``predict_transitions`` / ``transition_summary``: the
+per-step two-state posteriors of the same annotation), plus the data formats either side of it:
 ``readers.read_table`` (table -> length-bucketed ``all_tracks``) and ``simulate.sim_tracks``.  See DESIGN.md.
 """
 from . import readers, tracking  # noqa: F401
@@ -14,6 +15,8 @@ from .tracking import (  # noqa: F401
     get_params,
     param_fitting,
     predict_Bs,
+    predict_transitions,
+    transition_summary,
 )
 
 __version__ = "0.1.0"

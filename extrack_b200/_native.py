@@ -8,7 +8,7 @@ from __future__ import annotations
 
 import ctypes as C
 import os
-from typing import List, Optional, Sequence
+from typing import List, Optional, Sequence, Tuple
 
 import numpy as np
 
@@ -87,6 +87,7 @@ EXPORTS = (
     "xt_chunk_logp",
     "xt_plan_dump",
     "xt_predict",
+    "xt_predict_pairs",
     "xt_refine_positions",
     "xt_get_stats",
     "xt_seglen_hist",
@@ -140,6 +141,7 @@ def load_library() -> C.CDLL:
     lib.xt_chunk_logp.argtypes = [vp, i32, P(XtParams), P(dbl)]
     lib.xt_plan_dump.argtypes = [vp, i32, i32, P(i32), P(i32), P(i32), i32, P(dbl)]
     lib.xt_predict.argtypes = [vp, P(XtParams), P(vp)]
+    lib.xt_predict_pairs.argtypes = [vp, P(XtParams), P(vp), P(vp)]
     lib.xt_refine_positions.argtypes = [vp, P(XtParams), P(XtParams), P(vp), P(vp)]
     lib.xt_get_stats.argtypes = [vp, P(XtStats)]
     lib.xt_seglen_hist.argtypes = [vp, P(XtParams), P(dbl), P(dbl), i32, i32, vp, vp, P(i32)]
@@ -326,6 +328,15 @@ class Engine:
         ptrs = (C.c_void_p * len(outs))(*[o.ctypes.data for o in outs])
         self._check(self._lib.xt_predict(self._h, C.byref(p), ptrs))
         return outs
+
+    def predict_pairs(self, p: XtParams, nS: int) -> Tuple[List[np.ndarray], List[np.ndarray]]:
+        """``predict`` plus the two-slice posteriors [n, L - 1, nS, nS] per uploaded segment (``xt_predict_pairs``)."""
+        outs = [np.empty((n, L, nS), dtype=np.float64) for (L, n) in self.segments]
+        pairs = [np.empty((n, L - 1, nS, nS), dtype=np.float64) for (L, n) in self.segments]
+        ptrs = (C.c_void_p * len(outs))(*[o.ctypes.data for o in outs])
+        pptrs = (C.c_void_p * len(pairs))(*[o.ctypes.data for o in pairs])
+        self._check(self._lib.xt_predict_pairs(self._h, C.byref(p), ptrs, pptrs))
+        return outs, pairs
 
     def refine_positions(self, p_rev: XtParams, p_fwd: XtParams):
         """Refined positions [n, L, d] and their standard deviations [n, L] per uploaded segment (every segment

@@ -13,6 +13,12 @@
 //     pred[s][label_s(c)] += a_child[c];  a_parent[p] = sum_r a_child[pK + r]
 //     a_child(step s-1)[c'] = a_parent(step s)[gid[c']] * w[c'] / sum_group w
 // The history labels keep the reference's int8 wrap (:543).  nb_substeps is 1 (:839).
+// With PAIRS the same sweep also yields the two-slice posteriors (the Baum-Welch "xi"): the newest history row of a
+// group q of the fusion at step s-1 is the weighted mixture of its members' labels, so with v_q[j] = mass of q's
+// children at step s that carry label j,
+//     pair[s-1][label(c')][j] += w[c'] * v_q[j]   for every member c' of q (normalised weight w[c'])
+// and the initial sequences give pair[0] directly.  This equals carrying a pair history through the reference's
+// expansions and fusions (oracle/pair_oracle.py).
 #pragma once
 #include "xt_common.cuh"
 #include "xt_plan.cuh"
@@ -46,7 +52,12 @@ struct K3Args {
   // field-of-view / bleaching terms, initial fractions added at the end; instead of posteriors it stores, for every
   // step, (mean[d], std[KS], log-weight, newest state) of every surviving sequence of every track
   int32_t rev;           // 1: consume the localisations from the last to the first (get_LC_Km_Ks' own order)
-  double* dump;          // [n_tracks][L - 1 entries][capD][d + KS + 2] doubles, per chunk at dump_off[chunk]
+  union {
+    double* dump;        // [n_tracks][L - 1 entries][capD][d + KS + 2] doubles, per chunk at dump_off[chunk]
+    // PAIRS instantiation (predict_transitions, never REFINE): two-slice posteriors P(s_k = i, s_k+1 = j | track),
+    // [sum over tracks of (L - 1)][nS][nS] in forward time; a track's rows start at loc_off - trk_off + t (L - 1)
+    double* pairs;
+  };
   const int64_t* dump_off;
   int32_t* ent_n;        // [n_chunks][maxL]: sequences per entry (written by the chunk's first track)
   int32_t capD;
@@ -107,10 +118,61 @@ static __device__ K3_NI double k3_log(double x) { return log(x); }
 static __device__ K3_NI double k3_exp(double x) { return exp(x); }
 static __device__ K3_NI bool k3_div_lt(double a, double s, double th) { return __ddiv_rn(a, s) < th; }
 
-template <int D, int KS, bool VAR = false, bool FOLLOW = false, bool REFINE = false, int NSC = 0>
+// Pair row `row` (states at localisations row, row + 1) of one track into po[nS][nS], from the n sequences c' of level
+// `row` and av = the posterior of the children of level row + 1 (child q*nS + r of sequence / group q).  rw / rg: the
+// fusion records of level `row` (normalised weight, group); nullptr at level 1, whose sequences are the initial ones
+// (newest state c' % nS, unfused: weight 1, parent of the children c' itself).
+template <int NSC>
+static __device__ __forceinline__ void k3_emit_pairs(double* po, const double* av, int n, const double* rw, const uint16_t* rg,
+                                                     int nS, bool wrap, int lane) {
+  if constexpr (NSC == 2 || NSC == 4) {
+    // the label of c' is the residue of its lane (also c' % nS at level 1), and child q*NSC + j carries label j
+    double acc[NSC];
+#pragma unroll
+    for (int j = 0; j < NSC; ++j) acc[j] = 0.0;
+    #pragma unroll 1
+    for (int c = lane; c < n; c += 32) {
+      const double w = rw ? rw[c] : 1.0;
+      const int q = rw ? (int)rg[c] : c;
+#pragma unroll
+      for (int j = 0; j < NSC; ++j) acc[j] += w * av[q * NSC + j];
+    }
+#pragma unroll
+    for (int j = 0; j < NSC; ++j) {
+#pragma unroll
+      for (int o2 = 16; o2 >= NSC; o2 >>= 1) acc[j] += __shfl_xor_sync(0xffffffffu, acc[j], o2);
+    }
+    if (lane < NSC) {
+#pragma unroll
+      for (int j = 0; j < NSC; ++j) po[lane * NSC + j] = acc[j];
+    }
+  } else {
+    for (int i = 0; i < nS; ++i) {
+      for (int j = 0; j < nS; ++j) {
+        double acc = 0.0;
+        #pragma unroll 1
+        for (int c = lane; c < n; c += 32) {
+          if ((rw ? xt_label(c, nS, wrap) : c % nS) != i) continue;
+          const int q = rw ? (int)rg[c] : c;
+          double v = 0.0;
+          #pragma unroll 1
+          for (int r = 0; r < nS; ++r)
+            if (xt_label(q * nS + r, nS, wrap) == j) v += av[q * nS + r];
+          acc += (rw ? rw[c] : 1.0) * v;
+        }
+#pragma unroll
+        for (int o2 = 16; o2 > 0; o2 >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o2);
+        if (lane == 0) po[i * nS + j] = acc;
+      }
+    }
+  }
+}
+
+template <int D, int KS, bool VAR = false, bool FOLLOW = false, bool REFINE = false, int NSC = 0, bool PAIRS = false>
 __global__ void __launch_bounds__(32 * XT_K3_WARPS, XT_K3_MIN_CTAS) k3_predict(const K3Args a, const __grid_constant__ xt_params P) {
   static_assert(!(VAR && FOLLOW), "shared plans are built for scalar LocErr / dt models");
   static_assert(!REFINE || FOLLOW, "the refinement recursion follows the bucket's shared plan");
+  static_assert(!(REFINE && PAIRS), "the refinement stores no posteriors");
   // NSC > 0: the number of states is the compile-time constant NSC and the hot scratch is known to be in shared memory
   // (32-bit shared-memory addressing, shifts / multiply-shifts instead of integer divisions); NSC == 0: both at run time
   constexpr bool HOT = NSC > 0;
@@ -686,6 +748,11 @@ __global__ void __launch_bounds__(32 * XT_K3_WARPS, XT_K3_MIN_CTAS) k3_predict(c
           if (lane + 32 < nCprev) { w1 = rwp[lane + 32]; q1 = rgp[lane + 32]; }
         }
         emit_row(step, aC, nC, 0);  // newest row of this level: forward-time index = step
+        if constexpr (PAIRS) {
+          double* po = a.pairs + ((size_t)(ck.loc_off - ck.trk_off) + (size_t)t * (L - 1) + step - 1) * nS * nS;
+          if (step > 2) k3_emit_pairs<NSC>(po, aC, nCprev, rwp, rgp, nS, wrap, lane);
+          else k3_emit_pairs<NSC>(po, aC, nS * nS, nullptr, nullptr, nS, wrap, lane);
+        }
         const int nPar = nC / K;
         for (int p = lane; p < nPar; p += 32) {
           double sacc = 0.0;
@@ -711,6 +778,10 @@ __global__ void __launch_bounds__(32 * XT_K3_WARPS, XT_K3_MIN_CTAS) k3_predict(c
       // initial sequences j = h0 + nS*h1: row 1 = h0 (newest of the two), row 0 = h1 (oldest)
       emit_row(1, init_src, nS * nS, 1);
       emit_row(0, init_src, nS * nS, 2);
+      if constexpr (PAIRS) {  // initial sequence c = h0 + nS*h1 is the pair (h1, h0): flat index h1*nS + h0 = c
+        double* po = a.pairs + ((size_t)(ck.loc_off - ck.trk_off) + (size_t)t * (L - 1)) * nS * nS;
+        for (int c = lane; c < nS * nS; c += 32) po[c] = init_src[c];
+      }
       __syncwarp();
     }
   }

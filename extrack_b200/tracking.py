@@ -645,8 +645,9 @@ def Proba_Cs(Cs, LocErr, ds, Fs, TrMat, pBL, isBL, cell_dims, nb_substeps, frame
 # --------------------------------------------------------------------------------------
 # state annotation (tracking.py:792-906)
 # --------------------------------------------------------------------------------------
-def _gather_predictions(preds_local, sorted_tracks, world, nb_states, nb_max=1):
-    """All ranks' slices of every bucket -> full arrays in input order (rank r holds rows predict_shard(n, r, world))."""
+def _gather_predictions(preds_local, sorted_tracks, world, nb_states, nb_max=1, pairs=False):
+    """All ranks' slices of every bucket -> full arrays in input order (rank r holds rows predict_shard(n, r, world)).
+    ``pairs``: the slices are two-slice posteriors [rows, L - 1, nb_states, nb_states]."""
     import torch
     import torch.distributed as dist
 
@@ -656,7 +657,8 @@ def _gather_predictions(preds_local, sorted_tracks, world, nb_states, nb_max=1):
         n, L = a.shape[0], a.shape[1]
         rows = [predict_shard(n, r, world, nb_max) for r in range(world)]
         pad = max(hi - lo for lo, hi in rows)
-        buf = torch.zeros((pad, L, nb_states), dtype=torch.float64, device=dev)
+        row_shape = (L - 1, nb_states, nb_states) if pairs else (L, nb_states)
+        buf = torch.zeros((pad,) + row_shape, dtype=torch.float64, device=dev)
         buf[: len(mine)] = torch.from_numpy(np.ascontiguousarray(mine)).to(dev)
         parts = [torch.empty_like(buf) for _ in range(world)]
         dist.all_gather(parts, buf)
@@ -686,6 +688,52 @@ def predict_Bs(all_tracks, dt, params, cell_dims=[1], nb_states=4, frame_len=5, 
     collective.  ``gather=True`` (default) reassembles the full dictionary on every rank in input
     order (one all-gather per bucket); ``gather=False`` returns only this rank's rows.
     """
+    return _annotate(all_tracks, dt, params, cell_dims, nb_states, frame_len, max_nb_states, threshold, input_LocErr, nb_max,
+                     gather, False)[0]
+
+
+def predict_transitions(all_tracks, dt, params, cell_dims=[1], nb_states=4, frame_len=5, max_nb_states=200, threshold=0.1,
+                        workers=1, input_LocErr=None, verbose=0, nb_max=1, gather=True):
+    """``predict_Bs`` plus the two-slice (transition) posteriors of the same recursion: ``(preds, pairs)``, two
+    ``{str(L): array}`` dictionaries.  ``preds[k]`` is ``predict_Bs``'s float64[n, L, nb_states];
+    ``pairs[k]`` is float64[n, L - 1, nb_states, nb_states] with ``pairs[k][t, i, a, b]`` = P(state a at localisation
+    i, state b at localisation i + 1 | track t), forward time.  ``pairs.sum(-1) == preds[:, :-1]`` and
+    ``pairs.sum(-2) == preds[:, 1:]`` to rounding.  The probability that track t switches state between localisations
+    i and i + 1 is ``1 - trace(pairs[t, i])``; ``transition_summary`` aggregates them.
+
+    Arguments, validation, ``nb_max`` rules and errors, ``torch.distributed`` sharding and ``gather`` are those of
+    ``predict_Bs`` (the pairs take one more all-gather per bucket).
+    """
+    return _annotate(all_tracks, dt, params, cell_dims, nb_states, frame_len, max_nb_states, threshold, input_LocErr, nb_max,
+                     gather, True)
+
+
+def transition_summary(preds, pairs):
+    """Switching statistics from ``predict_transitions``' outputs (host only).
+
+    Returns ``(expected, TrMat_emp)``: ``expected`` = ``{str(L): float64[n]}``, the expected number of state changes
+    of every track (sum over its steps of ``1 - trace(pairs)``); ``TrMat_emp`` = float64[nS, nS], the empirical
+    per-step transition matrix ``sum xi[i, j] / sum_(steps) P(s = i)`` over all steps of all tracks, to hold against
+    the fitted transition probabilities (rows sum to 1; a state never occupied gives a row of NaN)."""
+    expected = {}
+    num = den = None
+    for k, q in pairs.items():
+        q = np.asarray(q, dtype=np.float64)
+        nS = q.shape[-1]
+        expected[k] = (1.0 - np.trace(q, axis1=-2, axis2=-1)).sum(axis=1)
+        if num is None:
+            num, den = np.zeros((nS, nS)), np.zeros(nS)
+        num += q.sum(axis=(0, 1))
+        den += np.asarray(preds[k], dtype=np.float64)[:, :-1].sum(axis=(0, 1))
+    if num is None:
+        raise ValueError("no tracks")
+    with np.errstate(invalid="ignore", divide="ignore"):
+        return expected, num / den[:, None]
+
+
+def _annotate(all_tracks, dt, params, cell_dims, nb_states, frame_len, max_nb_states, threshold, input_LocErr, nb_max, gather,
+              with_pairs):
+    """Body of predict_Bs / predict_transitions: (preds, pairs or None) as {str(L): array} dictionaries."""
     sorted_tracks, l_list = _sorted_buckets(all_tracks)
     keys = [k for k in l_list if len(all_tracks[k]) > 0]
     sorted_LocErrs = [np.asarray(input_LocErr[k], dtype=np.float64) for k in keys] if input_LocErr is not None else None
@@ -703,8 +751,9 @@ def predict_Bs(all_tracks, dt, params, cell_dims=[1], nb_states=4, frame_len=5, 
     if len(Ds) != nb_states:
         raise ValueError("nb_states (%d) must equal the number of D parameters (%d)" % (nb_states, len(Ds)))
     out = {l: np.empty((0, int(l), nb_states)) for l in l_list}
+    out_pairs = {l: np.empty((0, int(l) - 1, nb_states, nb_states)) for l in l_list} if with_pairs else None
     if not sorted_tracks:
-        return out
+        return out, out_pairs
     for a in sorted_tracks:
         if a.shape[1] < 2:
             raise ValueError("minimal track length = 2, here track length = %s" % a.shape[1])
@@ -729,6 +778,7 @@ def predict_Bs(all_tracks, dt, params, cell_dims=[1], nb_states=4, frame_len=5, 
     mine = [b for b, (lo, hi) in enumerate(cuts) if hi > lo]
     loc = lambda arrs: [arrs[b][cuts[b][0]:cuts[b][1]] for b in mine] if arrs is not None else None
     preds_local = [np.empty((0, a.shape[1], nb_states)) for a in sorted_tracks]
+    pairs_local = [np.empty((0, a.shape[1] - 1, nb_states, nb_states)) for a in sorted_tracks]
     if mine:
         eng = _native.Engine(_default_device())
         try:
@@ -742,14 +792,24 @@ def predict_Bs(all_tracks, dt, params, cell_dims=[1], nb_states=4, frame_len=5, 
             if sorted_dt is not None:
                 t0 = np.concatenate([a[:, 0] for a in loc(sorted_dt)])
                 eng.set_stay_tables(True, *stay_tables(Ds, np.stack([t0, t0], 1), TrMat, pBL, cell_dims, nb_substeps))
-            for b, pr in zip(mine, eng.predict(p, nb_states)):
-                preds_local[b] = pr
+            if with_pairs:
+                prs, qrs = eng.predict_pairs(p, nb_states)
+                for b, pr, qr in zip(mine, prs, qrs):
+                    preds_local[b], pairs_local[b] = pr, qr
+            else:
+                for b, pr in zip(mine, eng.predict(p, nb_states)):
+                    preds_local[b] = pr
         finally:
             eng.close()
     preds = preds_local if (world == 1 or not gather) else _gather_predictions(preds_local, sorted_tracks, world, nb_states, nb_max)
     for a, pr in zip(sorted_tracks, preds):
         out[str(a.shape[1])] = pr
-    return out
+    if with_pairs:
+        pairs = (pairs_local if (world == 1 or not gather)
+                 else _gather_predictions(pairs_local, sorted_tracks, world, nb_states, nb_max, pairs=True))
+        for a, q in zip(sorted_tracks, pairs):
+            out_pairs[str(a.shape[1])] = q
+    return out, out_pairs
 
 
 # --------------------------------------------------------------------------------------

@@ -181,6 +181,14 @@ int xt_plan_dump(xt_ctx* ctx, int32_t chunk, int32_t step, int32_t* nB_in, int32
 int xt_predict(xt_ctx* ctx, const xt_params* p, double* const* out);
 
 /*
+ * State annotation with transition posteriors: xt_predict (same options, plans and errors, same out[s]) that also fills
+ * out_pairs[s] with double[n[s]][L[s] - 1][nS][nS], entry [t][k][i][j] = P(state i at localisation k, state j at
+ * localisation k + 1 | track t) in forward time (the two-slice posteriors of the same recursion; summing over j gives
+ * out[s][t][k], over i out[s][t][k + 1]).
+ */
+int xt_predict_pairs(xt_ctx* ctx, const xt_params* p, double* const* out, double* const* out_pairs);
+
+/*
  * Position refinement — replaces extrack/refined_localization.py:207-338 (get_pos_PDF + the weighted means of
  * position_refinement) for the uploaded tracks.  Upload every length bucket as ONE chunk (chunk_size >= its track
  * count): the reference hands whole buckets to get_LC_Km_Ks (:48-204), whose grouping plan comes from the bucket's first
