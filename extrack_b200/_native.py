@@ -88,6 +88,7 @@ EXPORTS = (
     "xt_plan_dump",
     "xt_predict",
     "xt_predict_pairs",
+    "xt_predict_residuals",
     "xt_refine_positions",
     "xt_get_stats",
     "xt_seglen_hist",
@@ -142,6 +143,7 @@ def load_library() -> C.CDLL:
     lib.xt_plan_dump.argtypes = [vp, i32, i32, P(i32), P(i32), P(i32), i32, P(dbl)]
     lib.xt_predict.argtypes = [vp, P(XtParams), P(vp)]
     lib.xt_predict_pairs.argtypes = [vp, P(XtParams), P(vp), P(vp)]
+    lib.xt_predict_residuals.argtypes = [vp, P(XtParams), P(vp), P(vp), P(vp)]
     lib.xt_refine_positions.argtypes = [vp, P(XtParams), P(XtParams), P(vp), P(vp)]
     lib.xt_get_stats.argtypes = [vp, P(XtStats)]
     lib.xt_seglen_hist.argtypes = [vp, P(XtParams), P(dbl), P(dbl), i32, i32, vp, vp, P(i32)]
@@ -337,6 +339,16 @@ class Engine:
         pptrs = (C.c_void_p * len(pairs))(*[o.ctypes.data for o in pairs])
         self._check(self._lib.xt_predict_pairs(self._h, C.byref(p), ptrs, pptrs))
         return outs, pairs
+
+    def predict_residuals(self, p: XtParams, nS: int) -> Tuple[List[np.ndarray], List[np.ndarray], List[np.ndarray]]:
+        """``predict`` plus the one-step-ahead log predictive densities [n, L] and PIT values [n, L, d] per uploaded
+        segment (``xt_predict_residuals``; localisation 0 is NaN)."""
+        outs = [np.empty((n, L, nS), dtype=np.float64) for (L, n) in self.segments]
+        lps = [np.empty((n, L), dtype=np.float64) for (L, n) in self.segments]
+        pits = [np.empty((n, L, self.d), dtype=np.float64) for (L, n) in self.segments]
+        arr = lambda xs: (C.c_void_p * len(xs))(*[o.ctypes.data for o in xs])
+        self._check(self._lib.xt_predict_residuals(self._h, C.byref(p), arr(outs), arr(lps), arr(pits)))
+        return outs, lps, pits
 
     def refine_positions(self, p_rev: XtParams, p_fwd: XtParams):
         """Refined positions [n, L, d] and their standard deviations [n, L] per uploaded segment (every segment

@@ -12,6 +12,8 @@ struct K3Args;
 struct K3SArgs;
 struct KRArgs;
 struct K4Args;
+// what a state-annotation launch writes next to the posteriors (selects the k3_predict instantiation)
+enum K3Out { K3_OUT_PREDS = 0, K3_OUT_PAIRS = 1, K3_OUT_RESID = 2 };
 
 #define XT_DISPATCH(D_, KS_, CALL)                                   \
   do {                                                               \
@@ -58,12 +60,14 @@ cudaError_t xt_launch_k2_f32(int d, int ks, const K2FArgs& a, const K2Tab& tab, 
 // first-generation linear-domain kernel / log-domain fallback (xt_replay_lin.cuh, xt_replay.cuh)
 cudaError_t xt_launch_k2_old(const K2Args& a, const xt_params& p, const K2Lin& lin, size_t smem, bool use_smem, int grid,
                              int wpc, cudaStream_t stream);
-// state annotation (xt_predict.cuh); with a.pairs set, the instantiation that also writes the two-slice posteriors
-cudaError_t xt_launch_k3(const K3Args& a, const xt_params& p, int grid, int nwarps, size_t smem, cudaStream_t stream);
-int xt_k3_regs(const xt_params& p, int hot_smem, bool pairs);  // registers per thread of the kernel xt_launch_k3 would launch
+// state annotation (xt_predict.cuh); `out`: the instantiation that also writes the two-slice posteriors (a.pairs) or the
+// residuals (a.resid)
+cudaError_t xt_launch_k3(const K3Args& a, const xt_params& p, int grid, int nwarps, size_t smem, cudaStream_t stream, K3Out out);
+int xt_k3_regs(const xt_params& p, int hot_smem, K3Out out);  // registers per thread of the kernel xt_launch_k3 would launch
 // ... with plans shared by the nb_max tracks of a chunk (xt_predict_shared.cuh): the plans, then the annotation along them
 cudaError_t xt_launch_k3_shared_plan(const K3SArgs& a, const xt_params& p, int grid, cudaStream_t stream);
-cudaError_t xt_launch_k3_follow(const K3Args& a, const xt_params& p, int grid, int nwarps, size_t smem, cudaStream_t stream);
+cudaError_t xt_launch_k3_follow(const K3Args& a, const xt_params& p, int grid, int nwarps, size_t smem, cudaStream_t stream,
+                                K3Out out);
 // position refinement (xt_refine.cuh): recursion that stores every step, combination of its two passes
 cudaError_t xt_launch_k3_refine(const K3Args& a, const xt_params& p, int grid, int nwarps, size_t smem, cudaStream_t stream);
 cudaError_t xt_launch_refine_combine(int d, int ks, const KRArgs& a, unsigned grid, cudaStream_t stream);

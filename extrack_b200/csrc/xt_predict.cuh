@@ -19,7 +19,15 @@
 //     pair[s-1][label(c')][j] += w[c'] * v_q[j]   for every member c' of q (normalised weight w[c'])
 // and the initial sequences give pair[0] directly.  This equals carrying a pair history through the reference's
 // expansions and fusions (oracle/pair_oracle.py).
+// With RESID the forward pass also yields the one-step-ahead predictive of every localisation c_k (k >= 1): at the step
+// that consumes c_k, every live sequence j (a child of the expansion, or a final sequence at the end of the track) has
+// the predictive Gaussian N(m_j, q_j) of c_k (its parent's mean, q_j = l2 + s2_j), the Gaussian term LC_j of c_k and
+// the log-weight A_j = (log-weight after the step) - LC_j.  The mixture over j gives
+//     logpred[k] = logsumexp_j(A_j + LC_j) - logsumexp_j(A_j)
+//     pit[k][x]  = sum_j softmax(A)_j Phi((c_k,x - m_j,x) / sqrt(q_j,kappa(x)))
+// m, q and LC are those of the parent, so they and Phi are evaluated once per parent (oracle/resid_oracle.py).
 #pragma once
+#include <math_constants.h>
 #include "xt_common.cuh"
 #include "xt_plan.cuh"
 
@@ -57,6 +65,9 @@ struct K3Args {
     // PAIRS instantiation (predict_transitions, never REFINE): two-slice posteriors P(s_k = i, s_k+1 = j | track),
     // [sum over tracks of (L - 1)][nS][nS] in forward time; a track's rows start at loc_off - trk_off + t (L - 1)
     double* pairs;
+    // RESID instantiation (predict_residuals, never REFINE nor PAIRS): {logpred, pit}, a device array of two pointers
+    // to [sum over tracks of L] and [sum over tracks of L][d] doubles in forward time, a track's rows at loc_off + t L
+    double* const* resid;
   };
   const int64_t* dump_off;
   int32_t* ent_n;        // [n_chunks][maxL]: sequences per entry (written by the chunk's first track)
@@ -168,11 +179,81 @@ static __device__ __forceinline__ void k3_emit_pairs(double* po, const double* a
   }
 }
 
-template <int D, int KS, bool VAR = false, bool FOLLOW = false, bool REFINE = false, int NSC = 0, bool PAIRS = false>
+// Residuals of one localisation cl (RESID): the n sequences p of buf (slot pitch `pitch`: mean [D], s2 [KS], log-weight at
+// component D + 2 KS) are the parents of nch sequences each, the r-th with A = log-weight + add(p, r).  Lane 0 writes
+// logpred to lp[0] and the PIT values to pit[0..D).
+template <int D, int KS, class AddF>
+static __device__ __forceinline__ void k3_emit_resid(double* lp, double* pit, const double* buf, int pitch, int n, int nch,
+                                                     const double* cl, const double* l2, AddF add, int lane) {
+  auto lc_of = [&](int p) {  // the Gaussian term of cl under the predictive of parent p
+    double lc = 0.0;
+#pragma unroll
+    for (int dim = 0; dim < D; ++dim) {
+      const int k = (KS == 1) ? 0 : dim;
+      const double q = buf[(D + k) * pitch + p] + l2[k];
+      const double df = cl[dim] - buf[dim * pitch + p];
+      lc += -0.5 * log(XT_TWO_PI * q) - df * df / (2.0 * q);
+    }
+    return lc;
+  };
+  double mA = -INFINITY, mB = -INFINITY;
+  #pragma unroll 1
+  for (int p = lane; p < n; p += 32) {
+    const double lc = lc_of(p), a0 = buf[(D + 2 * KS) * pitch + p];
+    #pragma unroll 1
+    for (int r = 0; r < nch; ++r) {
+      const double A = a0 + add(p, r);
+      mA = fmax(mA, A);
+      mB = fmax(mB, A + lc);
+    }
+  }
+#pragma unroll
+  for (int o2 = 16; o2 > 0; o2 >>= 1) {
+    mA = fmax(mA, __shfl_xor_sync(0xffffffffu, mA, o2));
+    mB = fmax(mB, __shfl_xor_sync(0xffffffffu, mB, o2));
+  }
+  double s0 = 0.0, s1 = 0.0, sx[D];
+#pragma unroll
+  for (int dim = 0; dim < D; ++dim) sx[dim] = 0.0;
+  #pragma unroll 1
+  for (int p = lane; p < n; p += 32) {
+    const double lc = lc_of(p), a0 = buf[(D + 2 * KS) * pitch + p];
+    double w = 0.0;  // softmax numerators of p's children
+    #pragma unroll 1
+    for (int r = 0; r < nch; ++r) {
+      const double A = a0 + add(p, r);
+      w += exp(A - mA);
+      s1 += exp(A + lc - mB);
+    }
+    s0 += w;
+#pragma unroll
+    for (int dim = 0; dim < D; ++dim) {
+      const int k = (KS == 1) ? 0 : dim;
+      const double q = buf[(D + k) * pitch + p] + l2[k];
+      sx[dim] += w * normcdf((cl[dim] - buf[dim * pitch + p]) / sqrt(q));
+    }
+  }
+#pragma unroll
+  for (int o2 = 16; o2 > 0; o2 >>= 1) {
+    s0 += __shfl_xor_sync(0xffffffffu, s0, o2);
+    s1 += __shfl_xor_sync(0xffffffffu, s1, o2);
+#pragma unroll
+    for (int dim = 0; dim < D; ++dim) sx[dim] += __shfl_xor_sync(0xffffffffu, sx[dim], o2);
+  }
+  if (lane == 0) {
+    lp[0] = (log(s1) + mB) - (log(s0) + mA);
+#pragma unroll
+    for (int dim = 0; dim < D; ++dim) pit[dim] = sx[dim] / s0;
+  }
+}
+
+template <int D, int KS, bool VAR = false, bool FOLLOW = false, bool REFINE = false, int NSC = 0, bool PAIRS = false,
+          bool RESID = false>
 __global__ void __launch_bounds__(32 * XT_K3_WARPS, XT_K3_MIN_CTAS) k3_predict(const K3Args a, const __grid_constant__ xt_params P) {
   static_assert(!(VAR && FOLLOW), "shared plans are built for scalar LocErr / dt models");
   static_assert(!REFINE || FOLLOW, "the refinement recursion follows the bucket's shared plan");
   static_assert(!(REFINE && PAIRS), "the refinement stores no posteriors");
+  static_assert(!(REFINE && RESID) && !(PAIRS && RESID), "the residuals share the output pointer of the other modes");
   // NSC > 0: the number of states is the compile-time constant NSC and the hot scratch is known to be in shared memory
   // (32-bit shared-memory addressing, shifts / multiply-shifts instead of integer divisions); NSC == 0: both at run time
   constexpr bool HOT = NSC > 0;
@@ -235,6 +316,16 @@ __global__ void __launch_bounds__(32 * XT_K3_WARPS, XT_K3_MIN_CTAS) k3_predict(c
       const double* Cp = a.soa + ck.xyz_off + t;
       const size_t npad = (size_t)ck.nTpad;
       double* out = a.pred + ((size_t)ck.loc_off + (size_t)t * L) * nS;
+      // RESID: this track's logpred [L] and pit [L][D] start at localisation loc_off + t L; the first localisation has no
+      // predictive
+      if constexpr (RESID) {
+        const size_t row0 = (size_t)ck.loc_off + (size_t)t * L;
+        if (lane == 0) {
+          a.resid[0][row0] = CUDART_NAN;
+#pragma unroll
+          for (int dim = 0; dim < D; ++dim) a.resid[1][row0 * D + dim] = CUDART_NAN;
+        }
+      }
       int errc = 0;
       const bool rev = REFINE && a.rev;
 #define LROW(j) (rev ? (L - 1 - (j)) : (j))  // localisation consumed j-th
@@ -351,6 +442,11 @@ __global__ void __launch_bounds__(32 * XT_K3_WARPS, XT_K3_MIN_CTAS) k3_predict(c
         }
         if (nC > P.max_nb_states) th = __dmul_rn(th, 1.2);
         __syncwarp();
+        if constexpr (RESID) {  // localisation step - 1 under the K children of every parent
+          const size_t row = (size_t)ck.loc_off + (size_t)t * L + step - 1;
+          k3_emit_resid<D, KS>(a.resid[0] + row, a.resid[1] + row * D, bufP, capP, nP, K, cl, l2,
+                               [&](int p, int r) { return P.LT[r + K * curP[p]] + (stay ? Lps[r] : 0.0); }, lane);
+        }
         if (step == L - 1) {  // last step: no fusion (tracking.py:591)
           nP = nC;
           LhP = LhC;
@@ -656,6 +752,11 @@ __global__ void __launch_bounds__(32 * XT_K3_WARPS, XT_K3_MIN_CTAS) k3_predict(c
 #pragma unroll
       for (int dim = 0; dim < D; ++dim) clast[dim] = Cp[(size_t)(LROW(L - 1) * D + dim) * npad];
       if (VAR) var_row(L - 1);
+      if constexpr (RESID) {  // the last localisation under the final sequences (the bleaching end sums its heads in Lsm)
+        const size_t row = (size_t)ck.loc_off + (size_t)t * L + L - 1;
+        k3_emit_resid<D, KS>(a.resid[0] + row, a.resid[1] + row * D, FB, fbs, nP, 1, clast, l2,
+                             [&](int c, int) { return ck.isBL ? Lsm[c % nS] : 0.0; }, lane);
+      }
       double vmax = -INFINITY;
       #pragma unroll 1
       for (int c = lane; c < nP; c += 32) {

@@ -645,9 +645,9 @@ def Proba_Cs(Cs, LocErr, ds, Fs, TrMat, pBL, isBL, cell_dims, nb_substeps, frame
 # --------------------------------------------------------------------------------------
 # state annotation (tracking.py:792-906)
 # --------------------------------------------------------------------------------------
-def _gather_predictions(preds_local, sorted_tracks, world, nb_states, nb_max=1, pairs=False):
+def _gather_predictions(preds_local, sorted_tracks, world, row_shape, nb_max=1):
     """All ranks' slices of every bucket -> full arrays in input order (rank r holds rows predict_shard(n, r, world)).
-    ``pairs``: the slices are two-slice posteriors [rows, L - 1, nb_states, nb_states]."""
+    ``row_shape(L)``: the shape of one track's entry in the slices of a bucket of length L."""
     import torch
     import torch.distributed as dist
 
@@ -657,8 +657,7 @@ def _gather_predictions(preds_local, sorted_tracks, world, nb_states, nb_max=1, 
         n, L = a.shape[0], a.shape[1]
         rows = [predict_shard(n, r, world, nb_max) for r in range(world)]
         pad = max(hi - lo for lo, hi in rows)
-        row_shape = (L - 1, nb_states, nb_states) if pairs else (L, nb_states)
-        buf = torch.zeros((pad,) + row_shape, dtype=torch.float64, device=dev)
+        buf = torch.zeros((pad,) + row_shape(L), dtype=torch.float64, device=dev)
         buf[: len(mine)] = torch.from_numpy(np.ascontiguousarray(mine)).to(dev)
         parts = [torch.empty_like(buf) for _ in range(world)]
         dist.all_gather(parts, buf)
@@ -689,7 +688,7 @@ def predict_Bs(all_tracks, dt, params, cell_dims=[1], nb_states=4, frame_len=5, 
     order (one all-gather per bucket); ``gather=False`` returns only this rank's rows.
     """
     return _annotate(all_tracks, dt, params, cell_dims, nb_states, frame_len, max_nb_states, threshold, input_LocErr, nb_max,
-                     gather, False)[0]
+                     gather, "preds")[0]
 
 
 def predict_transitions(all_tracks, dt, params, cell_dims=[1], nb_states=4, frame_len=5, max_nb_states=200, threshold=0.1,
@@ -705,7 +704,27 @@ def predict_transitions(all_tracks, dt, params, cell_dims=[1], nb_states=4, fram
     ``predict_Bs`` (the pairs take one more all-gather per bucket).
     """
     return _annotate(all_tracks, dt, params, cell_dims, nb_states, frame_len, max_nb_states, threshold, input_LocErr, nb_max,
-                     gather, True)
+                     gather, "pairs")
+
+
+def predict_residuals(all_tracks, dt, params, cell_dims=[1], nb_states=4, frame_len=5, max_nb_states=200, threshold=0.1,
+                      workers=1, input_LocErr=None, verbose=0, nb_max=1, gather=True):
+    """``predict_Bs`` plus the one-step-ahead residuals of the same recursion: ``(preds, logpred, pit)``, three
+    ``{str(L): array}`` dictionaries.  ``preds[k]`` is ``predict_Bs``'s float64[n, L, nb_states].
+
+    At the step that consumes localisation ``c_i`` (i >= 1), the live state sequences of the recursion form a Gaussian
+    mixture: the model's predictive distribution of ``c_i`` given ``c_0 .. c_i-1``.  ``logpred[k]`` is float64[n, L]:
+    the log density of that mixture at ``c_i``.  A mislinked localisation, or a jump no state explains, is a deep
+    minimum inside its track.  ``pit[k]`` is float64[n, L, d]: the mixture's cumulative distribution at ``c_i``, per
+    dimension (probability integral transform).  When the model describes the data these values are Uniform(0, 1); a
+    skewed histogram shows where it does not (for example a missing state).  Localisation 0 has no predictive: its
+    entries are NaN.
+
+    Arguments, validation, ``nb_max`` rules and errors, ``torch.distributed`` sharding and ``gather`` are those of
+    ``predict_Bs`` (logpred and pit take one more all-gather per bucket each).
+    """
+    return _annotate(all_tracks, dt, params, cell_dims, nb_states, frame_len, max_nb_states, threshold, input_LocErr, nb_max,
+                     gather, "resid")
 
 
 def transition_summary(preds, pairs):
@@ -732,8 +751,9 @@ def transition_summary(preds, pairs):
 
 
 def _annotate(all_tracks, dt, params, cell_dims, nb_states, frame_len, max_nb_states, threshold, input_LocErr, nb_max, gather,
-              with_pairs):
-    """Body of predict_Bs / predict_transitions: (preds, pairs or None) as {str(L): array} dictionaries."""
+              kind):
+    """Body of predict_Bs ("preds"), predict_transitions ("pairs") and predict_residuals ("resid"): the posteriors and
+    the arrays of that output kind, each as a {str(L): array} dictionary."""
     sorted_tracks, l_list = _sorted_buckets(all_tracks)
     keys = [k for k in l_list if len(all_tracks[k]) > 0]
     sorted_LocErrs = [np.asarray(input_LocErr[k], dtype=np.float64) for k in keys] if input_LocErr is not None else None
@@ -750,10 +770,16 @@ def _annotate(all_tracks, dt, params, cell_dims, nb_states, frame_len, max_nb_st
     loc, Ds, Fs, TrMat, pBL = _extract_scalars(params, nb_substeps)
     if len(Ds) != nb_states:
         raise ValueError("nb_states (%d) must equal the number of D parameters (%d)" % (nb_states, len(Ds)))
-    out = {l: np.empty((0, int(l), nb_states)) for l in l_list}
-    out_pairs = {l: np.empty((0, int(l) - 1, nb_states, nb_states)) for l in l_list} if with_pairs else None
+    d = next((np.shape(a)[2] for a in all_tracks.values() if np.ndim(a) == 3), 0)
+    # one track's entry of every returned array, by bucket length
+    row_shapes = [lambda L: (L, nb_states)] + {
+        "preds": [],
+        "pairs": [lambda L: (L - 1, nb_states, nb_states)],
+        "resid": [lambda L: (L,), lambda L: (L, d)],
+    }[kind]
+    outs = [{l: np.empty((0,) + rs(int(l))) for l in l_list} for rs in row_shapes]
     if not sorted_tracks:
-        return out, out_pairs
+        return tuple(outs)
     for a in sorted_tracks:
         if a.shape[1] < 2:
             raise ValueError("minimal track length = 2, here track length = %s" % a.shape[1])
@@ -777,8 +803,7 @@ def _annotate(all_tracks, dt, params, cell_dims, nb_states, frame_len, max_nb_st
     cuts = [predict_shard(len(a), rank, world, nb_max) for a in sorted_tracks]
     mine = [b for b, (lo, hi) in enumerate(cuts) if hi > lo]
     loc = lambda arrs: [arrs[b][cuts[b][0]:cuts[b][1]] for b in mine] if arrs is not None else None
-    preds_local = [np.empty((0, a.shape[1], nb_states)) for a in sorted_tracks]
-    pairs_local = [np.empty((0, a.shape[1] - 1, nb_states, nb_states)) for a in sorted_tracks]
+    local = [[np.empty((0,) + rs(a.shape[1])) for a in sorted_tracks] for rs in row_shapes]
     if mine:
         eng = _native.Engine(_default_device())
         try:
@@ -792,24 +817,22 @@ def _annotate(all_tracks, dt, params, cell_dims, nb_states, frame_len, max_nb_st
             if sorted_dt is not None:
                 t0 = np.concatenate([a[:, 0] for a in loc(sorted_dt)])
                 eng.set_stay_tables(True, *stay_tables(Ds, np.stack([t0, t0], 1), TrMat, pBL, cell_dims, nb_substeps))
-            if with_pairs:
-                prs, qrs = eng.predict_pairs(p, nb_states)
-                for b, pr, qr in zip(mine, prs, qrs):
-                    preds_local[b], pairs_local[b] = pr, qr
+            if kind == "pairs":
+                res = eng.predict_pairs(p, nb_states)
+            elif kind == "resid":
+                res = eng.predict_residuals(p, nb_states)
             else:
-                for b, pr in zip(mine, eng.predict(p, nb_states)):
-                    preds_local[b] = pr
+                res = (eng.predict(p, nb_states),)
+            for lo, arrs in zip(local, res):
+                for b, x in zip(mine, arrs):
+                    lo[b] = x
         finally:
             eng.close()
-    preds = preds_local if (world == 1 or not gather) else _gather_predictions(preds_local, sorted_tracks, world, nb_states, nb_max)
-    for a, pr in zip(sorted_tracks, preds):
-        out[str(a.shape[1])] = pr
-    if with_pairs:
-        pairs = (pairs_local if (world == 1 or not gather)
-                 else _gather_predictions(pairs_local, sorted_tracks, world, nb_states, nb_max, pairs=True))
-        for a, q in zip(sorted_tracks, pairs):
-            out_pairs[str(a.shape[1])] = q
-    return out, out_pairs
+    for out, lo, rs in zip(outs, local, row_shapes):
+        full = lo if (world == 1 or not gather) else _gather_predictions(lo, sorted_tracks, world, rs, nb_max)
+        for a, x in zip(sorted_tracks, full):
+            out[str(a.shape[1])] = x
+    return tuple(outs)
 
 
 # --------------------------------------------------------------------------------------

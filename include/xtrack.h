@@ -189,6 +189,17 @@ int xt_predict(xt_ctx* ctx, const xt_params* p, double* const* out);
 int xt_predict_pairs(xt_ctx* ctx, const xt_params* p, double* const* out, double* const* out_pairs);
 
 /*
+ * State annotation with one-step-ahead residuals: xt_predict (same options, plans and errors, same out[s]) that also
+ * fills logpred[s] with double[n[s]][L[s]] and pit[s] with double[n[s]][L[s]][d].  For localisation k >= 1 of track t,
+ * the recursion's live sequences j at the step that consumes c_k form the predictive mixture sum_j w_j N(m_j, q_j) of
+ * c_k given c_0..c_k-1 (w = softmax of their log-weights without the Gaussian term of c_k):
+ *   logpred[t][k]   = log of that mixture's density at c_k
+ *   pit[t][k][x]    = sum_j w_j Phi((c_k,x - m_j,x) / sqrt(q_j,x))   (Uniform(0, 1) when the model is right)
+ * Entry k = 0 is NaN (no predictive for the first localisation).
+ */
+int xt_predict_residuals(xt_ctx* ctx, const xt_params* p, double* const* out, double* const* logpred, double* const* pit);
+
+/*
  * Position refinement — replaces extrack/refined_localization.py:207-338 (get_pos_PDF + the weighted means of
  * position_refinement) for the uploaded tracks.  Upload every length bucket as ONE chunk (chunk_size >= its track
  * count): the reference hands whole buckets to get_LC_Km_Ks (:48-204), whose grouping plan comes from the bucket's first
