@@ -3,7 +3,8 @@
 Only the hot path of ``extrack.tracking`` is provided: ``param_fitting`` / ``cum_Proba_Cs`` /
 ``Proba_Cs`` / ``predict_Bs`` and the parameter builders (plus ``predict_transitions`` / ``transition_summary``: the
 per-step two-state posteriors of the same annotation, and ``predict_residuals``: its one-step-ahead predictive
-densities and PIT values), plus the data formats either side of it:
+densities and PIT values, and ``predict_path`` / ``path_segments``: its most probable state paths and their dwell
+times), plus the data formats either side of it:
 ``readers.read_table`` (table -> length-bucketed ``all_tracks``) and ``simulate.sim_tracks``.  See DESIGN.md.
 """
 from . import readers, tracking  # noqa: F401
@@ -15,7 +16,9 @@ from .tracking import (  # noqa: F401
     get_2DSPT_params,
     get_params,
     param_fitting,
+    path_segments,
     predict_Bs,
+    predict_path,
     predict_residuals,
     predict_transitions,
     transition_summary,

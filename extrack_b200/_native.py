@@ -89,6 +89,7 @@ EXPORTS = (
     "xt_predict",
     "xt_predict_pairs",
     "xt_predict_residuals",
+    "xt_predict_path",
     "xt_refine_positions",
     "xt_get_stats",
     "xt_seglen_hist",
@@ -144,6 +145,7 @@ def load_library() -> C.CDLL:
     lib.xt_predict.argtypes = [vp, P(XtParams), P(vp)]
     lib.xt_predict_pairs.argtypes = [vp, P(XtParams), P(vp), P(vp)]
     lib.xt_predict_residuals.argtypes = [vp, P(XtParams), P(vp), P(vp), P(vp)]
+    lib.xt_predict_path.argtypes = [vp, P(XtParams), P(vp), P(vp), P(vp)]
     lib.xt_refine_positions.argtypes = [vp, P(XtParams), P(XtParams), P(vp), P(vp)]
     lib.xt_get_stats.argtypes = [vp, P(XtStats)]
     lib.xt_seglen_hist.argtypes = [vp, P(XtParams), P(dbl), P(dbl), i32, i32, vp, vp, P(i32)]
@@ -349,6 +351,16 @@ class Engine:
         arr = lambda xs: (C.c_void_p * len(xs))(*[o.ctypes.data for o in xs])
         self._check(self._lib.xt_predict_residuals(self._h, C.byref(p), arr(outs), arr(lps), arr(pits)))
         return outs, lps, pits
+
+    def predict_path(self, p: XtParams, nS: int) -> Tuple[List[np.ndarray], List[np.ndarray], List[np.ndarray]]:
+        """``predict`` plus the MAP state paths int8[n, L] and their log posterior probabilities float64[n] per uploaded
+        segment (``xt_predict_path``)."""
+        outs = [np.empty((n, L, nS), dtype=np.float64) for (L, n) in self.segments]
+        paths = [np.empty((n, L), dtype=np.int8) for (L, n) in self.segments]
+        logps = [np.empty(n, dtype=np.float64) for (L, n) in self.segments]
+        arr = lambda xs: (C.c_void_p * len(xs))(*[o.ctypes.data for o in xs])
+        self._check(self._lib.xt_predict_path(self._h, C.byref(p), arr(outs), arr(paths), arr(logps)))
+        return outs, paths, logps
 
     def refine_positions(self, p_rev: XtParams, p_fwd: XtParams):
         """Refined positions [n, L, d] and their standard deviations [n, L] per uploaded segment (every segment

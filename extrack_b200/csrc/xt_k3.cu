@@ -5,32 +5,35 @@
 #include "xt_refine.cuh"
 
 // The own-plan annotation kernel of a model: scalar models with 2 or 3 states and the hot scratch in shared memory get
-// the instantiation with the number of states fixed at compile time (NSC), everything else the generic one.  `out`: the
-// instantiation that also writes the two-slice posteriors (K3Args::pairs) or the residuals (K3Args::resid).
+// the instantiation with the number of states fixed at compile time (NSC), everything else the generic one.  `OUT`: the
+// instantiation that also writes the two-slice posteriors (K3Args::pairs), the residuals (K3Args::resid) or the MAP
+// paths (K3Args::path).
 using K3Kern = void (*)(const K3Args, const xt_params);
 struct K3Pick {
   K3Kern kern;
   unsigned long long* smem_ok;
 };
-template <int D, int KS, bool VAR, int NSC, bool PAIRS, bool RESID>
+template <int D, int KS, bool VAR, int NSC, K3Out OUT>
 static K3Pick k3_one() {
   static unsigned long long smem_ok = 0;
-  return K3Pick{k3_predict<D, KS, VAR, false, false, NSC, PAIRS, RESID>, &smem_ok};
+  return K3Pick{k3_predict<D, KS, VAR, false, false, NSC, OUT == K3_OUT_PAIRS, OUT == K3_OUT_RESID, OUT == K3_OUT_PATH>,
+                &smem_ok};
 }
-template <int D, int KS, bool PAIRS, bool RESID>
+template <int D, int KS, K3Out OUT>
 static K3Pick k3_pick_nsc(bool var, int nsc) {
-  return var ? k3_one<D, KS, true, 0, PAIRS, RESID>()
-             : (nsc == 2 ? k3_one<D, KS, false, 2, PAIRS, RESID>()
-                         : (nsc == 3 ? k3_one<D, KS, false, 3, PAIRS, RESID>() : k3_one<D, KS, false, 0, PAIRS, RESID>()));
+  return var ? k3_one<D, KS, true, 0, OUT>()
+             : (nsc == 2 ? k3_one<D, KS, false, 2, OUT>()
+                         : (nsc == 3 ? k3_one<D, KS, false, 3, OUT>() : k3_one<D, KS, false, 0, OUT>()));
 }
 static K3Pick k3_pick(const xt_params& p, int hot_smem, K3Out out) {
   K3Pick k{nullptr, nullptr};
   const bool var = xt_is_var(&p);
   const int nsc = (!var && hot_smem && (p.nS == 2 || p.nS == 3)) ? p.nS : 0;
 #define PICK_K3(D_, KS_)                                                         \
-  k = out == K3_OUT_PAIRS   ? k3_pick_nsc<D_, KS_, true, false>(var, nsc)        \
-      : out == K3_OUT_RESID ? k3_pick_nsc<D_, KS_, false, true>(var, nsc)        \
-                            : k3_pick_nsc<D_, KS_, false, false>(var, nsc)
+  k = out == K3_OUT_PAIRS   ? k3_pick_nsc<D_, KS_, K3_OUT_PAIRS>(var, nsc)       \
+      : out == K3_OUT_RESID ? k3_pick_nsc<D_, KS_, K3_OUT_RESID>(var, nsc)       \
+      : out == K3_OUT_PATH  ? k3_pick_nsc<D_, KS_, K3_OUT_PATH>(var, nsc)        \
+                            : k3_pick_nsc<D_, KS_, K3_OUT_PREDS>(var, nsc)
   XT_DISPATCH(p.d, p.n_loc, PICK_K3);
 #undef PICK_K3
   return k;
@@ -66,9 +69,9 @@ cudaError_t xt_launch_k3_shared_plan(const K3SArgs& a, const xt_params& p, int g
 #undef CALL_K3S
   return e;
 }
-template <int D, int KS, bool PAIRS, bool RESID>
+template <int D, int KS, K3Out OUT>
 static cudaError_t launch_k3f(const K3Args& a, const xt_params& p, int grid, int nwarps, size_t smem, cudaStream_t stream) {
-  auto kern = k3_predict<D, KS, false, true, false, 0, PAIRS, RESID>;
+  auto kern = k3_predict<D, KS, false, true, false, 0, OUT == K3_OUT_PAIRS, OUT == K3_OUT_RESID, OUT == K3_OUT_PATH>;
   static unsigned long long smem_ok = 0;
   cudaError_t e = xt_allow_smem(kern, smem, &smem_ok);
   if (e != cudaSuccess) return e;
@@ -78,10 +81,11 @@ static cudaError_t launch_k3f(const K3Args& a, const xt_params& p, int grid, int
 cudaError_t xt_launch_k3_follow(const K3Args& a, const xt_params& p, int grid, int nwarps, size_t smem, cudaStream_t stream,
                                 K3Out out) {
   cudaError_t e = cudaSuccess;
-#define CALL_K3F(D_, KS_)                                                                                \
-  e = out == K3_OUT_PAIRS   ? launch_k3f<D_, KS_, true, false>(a, p, grid, nwarps, smem, stream)       \
-      : out == K3_OUT_RESID ? launch_k3f<D_, KS_, false, true>(a, p, grid, nwarps, smem, stream)       \
-                            : launch_k3f<D_, KS_, false, false>(a, p, grid, nwarps, smem, stream)
+#define CALL_K3F(D_, KS_)                                                                                  \
+  e = out == K3_OUT_PAIRS   ? launch_k3f<D_, KS_, K3_OUT_PAIRS>(a, p, grid, nwarps, smem, stream)        \
+      : out == K3_OUT_RESID ? launch_k3f<D_, KS_, K3_OUT_RESID>(a, p, grid, nwarps, smem, stream)        \
+      : out == K3_OUT_PATH  ? launch_k3f<D_, KS_, K3_OUT_PATH>(a, p, grid, nwarps, smem, stream)         \
+                            : launch_k3f<D_, KS_, K3_OUT_PREDS>(a, p, grid, nwarps, smem, stream)
   XT_DISPATCH(p.d, p.n_loc, CALL_K3F);
 #undef CALL_K3F
   return e;

@@ -26,6 +26,16 @@
 //     logpred[k] = logsumexp_j(A_j + LC_j) - logsumexp_j(A_j)
 //     pit[k][x]  = sum_j softmax(A)_j Phi((c_k,x - m_j,x) / sqrt(q_j,kappa(x)))
 // m, q and LC are those of the parent, so they and Phi are evaluated once per parent (oracle/resid_oracle.py).
+// With PATH the forward pass also yields the most probable state path (MAP / Viterbi path) of the lattice above: a route
+// from an initial to a final sequence has the weight softmax(LP)_final * prod of the merge weights w along it, the
+// routes' weights sum to 1 and the backward sweep sums them by label.  Every sequence carries a score V updated like its
+// LP, except that a fusion sets its group's V to the *maximum* of the members' V (LP: their log-sum-exp); the argmax
+// member (ties: the first in member order) is recorded per group and level (recArg).  The final choice is the argmax of
+// V + the end-of-track term of LP (the bleaching end's Lsum included; ties: the lowest index), and one lane backtracks
+// along recArg and the implicit parents c / K.  The labels are those of the posteriors (the int8 wrap included) and
+//     path_logp = V* - logsumexp(final LP) = log(weight of the heaviest route)
+// by telescoping.  Without fusion V = LP, so the path is the exact argmax over the state sequences
+// (oracle/path_oracle.py).
 #pragma once
 #include <math_constants.h>
 #include "xt_common.cuh"
@@ -68,6 +78,10 @@ struct K3Args {
     // RESID instantiation (predict_residuals, never REFINE nor PAIRS): {logpred, pit}, a device array of two pointers
     // to [sum over tracks of L] and [sum over tracks of L][d] doubles in forward time, a track's rows at loc_off + t L
     double* const* resid;
+    // PATH instantiation (predict_path, never REFINE, PAIRS nor RESID): {labels, path_logp}, a device array of two
+    // pointers to int8_t[sum over tracks of L] in forward time (a track's labels at loc_off + t L) and double[n_tracks]
+    // (a track's entry at trk_off + t)
+    void* const* path;
   };
   const int64_t* dump_off;
   int32_t* ent_n;        // [n_chunks][maxL]: sequences per entry (written by the chunk's first track)
@@ -82,6 +96,29 @@ struct K3Layout {
   size_t bufP, bufC, histP, histN, codeP, codeC, aC, aP, gid, order, goff, curP, hot_total;
   size_t recW, recN, recGid, cold_total;
 };
+// PATH instantiation: its own regions after the hot and the cold part of the other modes' layout `l`, and the totals
+// that include them
+struct K3PathLayout {
+  size_t vP, vC, hot_total;  // path scores of the parents / groups [cap / nS + 1] and of the children [cap]
+  size_t recArg, cold_total; // uint16[maxL][cap / nS + 1]: argmax member of every group of every fused step
+};
+__host__ __device__ inline K3PathLayout k3_path_layout(const K3Layout& l, int cap, int nS, int maxL) {
+  K3PathLayout q;
+  size_t o = l.hot_total;
+  q.vP = o;     o += cap / nS + 1;
+  q.vC = o;     o += cap;
+  q.hot_total = (o + 1) & ~(size_t)1;
+  q.recArg = l.cold_total;
+  q.cold_total = l.cold_total + ((size_t)maxL * (cap / nS + 1) + 3) / 4;
+  return q;
+}
+// The PATH arrays of one warp (hot part at `base`, cold part at `cold`)
+struct K3PathPtrs {
+  double* vP;        // path scores V of the parents / groups [cap / nS + 1]
+  double* vC;        // ... of the children [cap]
+  uint16_t* recArg;  // [maxL][cap / nS + 1]: argmax member of every group of every fused step
+};
+template <bool PATH = false>
 __host__ __device__ inline K3Layout k3_layout(int cap, int CO, int fl, int nS, int maxL) {
   K3Layout l;
   size_t o = 0;
@@ -106,7 +143,16 @@ __host__ __device__ inline K3Layout k3_layout(int cap, int CO, int fl, int nS, i
   l.recW = o;   o += (size_t)maxL * cap;
   l.recGid = o; o += ((size_t)maxL * cap + 3) / 4;  // uint16[maxL][cap]
   l.cold_total = o + 4;
+  if constexpr (PATH) {
+    const K3PathLayout q = k3_path_layout(l, cap, nS, maxL);
+    l.hot_total = q.hot_total;
+    l.cold_total = q.cold_total;
+  }
   return l;
+}
+static __device__ __forceinline__ K3PathPtrs k3_path_ptrs(double* base, double* cold, int cap, int CO, int fl, int nS, int maxL) {
+  const K3PathLayout q = k3_path_layout(k3_layout(cap, CO, fl, nS, maxL), cap, nS, maxL);
+  return K3PathPtrs{base + q.vP, base + q.vC, (uint16_t*)(cold + q.recArg)};
 }
 
 // The annotation kernel is sensitive to instruction fetch (ncu: 32 % of the stall samples were "no instruction" with
@@ -248,12 +294,13 @@ static __device__ __forceinline__ void k3_emit_resid(double* lp, double* pit, co
 }
 
 template <int D, int KS, bool VAR = false, bool FOLLOW = false, bool REFINE = false, int NSC = 0, bool PAIRS = false,
-          bool RESID = false>
+          bool RESID = false, bool PATH = false>
 __global__ void __launch_bounds__(32 * XT_K3_WARPS, XT_K3_MIN_CTAS) k3_predict(const K3Args a, const __grid_constant__ xt_params P) {
   static_assert(!(VAR && FOLLOW), "shared plans are built for scalar LocErr / dt models");
   static_assert(!REFINE || FOLLOW, "the refinement recursion follows the bucket's shared plan");
   static_assert(!(REFINE && PAIRS), "the refinement stores no posteriors");
   static_assert(!(REFINE && RESID) && !(PAIRS && RESID), "the residuals share the output pointer of the other modes");
+  static_assert(!(PATH && (REFINE || PAIRS || RESID)), "the MAP paths share the output pointer of the other modes");
   // NSC > 0: the number of states is the compile-time constant NSC and the hot scratch is known to be in shared memory
   // (32-bit shared-memory addressing, shifts / multiply-shifts instead of integer divisions); NSC == 0: both at run time
   constexpr bool HOT = NSC > 0;
@@ -273,7 +320,7 @@ __global__ void __launch_bounds__(32 * XT_K3_WARPS, XT_K3_MIN_CTAS) k3_predict(c
   };
 
   // ---- per-warp scratch carve-up ----
-  const K3Layout lay = k3_layout(cap, CO, fl, nS, a.maxL);
+  const K3Layout lay = k3_layout<PATH>(cap, CO, fl, nS, a.maxL);
   double* cold = a.scratch + (size_t)(blockIdx.x * nwarps + warp) * a.warp_scratch;
   double* base;
   if constexpr (HOT) base = k3_smem + warp * (int)lay.hot_total;
@@ -292,6 +339,9 @@ __global__ void __launch_bounds__(32 * XT_K3_WARPS, XT_K3_MIN_CTAS) k3_predict(c
   int* recN = (int*)(base + (int)lay.recN);       // children per fused step
   double* recW = cold + lay.recW;                 // [maxL][cap]
   uint16_t* recGid = (uint16_t*)(cold + lay.recGid);
+  // PATH: its arrays (K3PathPtrs) are fetched inside the PATH-only blocks, so that the other instantiations compile to
+  // exactly the code they had without this mode
+#define K3_PATH_PTRS const K3PathPtrs pa = k3_path_ptrs(base, cold, cap, CO, fl, nS, a.maxL)
 
   const int capP = cap / nS + 1;  // parent / group slots
 #define BP(slot, comp) bufP[(comp) * capP + (slot)]
@@ -366,6 +416,10 @@ __global__ void __launch_bounds__(32 * XT_K3_WARPS, XT_K3_MIN_CTAS) k3_predict(c
           e0[D + KS] = BP(c, D + 2 * KS);
           e0[D + KS + 1] = (double)(c % nS);
         }
+        if constexpr (PATH) {
+          K3_PATH_PTRS;
+          pa.vP[c] = BP(c, D + 2 * KS);
+        }
         curP[c] = c % nS;
         const int d0 = c % nS, d1 = c / nS;
         codeP[c] = (unsigned long long)d0 | ((unsigned long long)d1 << bits);
@@ -437,6 +491,10 @@ __global__ void __launch_bounds__(32 * XT_K3_WARPS, XT_K3_MIN_CTAS) k3_predict(c
           double add = __dadd_rn(P.LT[head], __dsub_rn(logs, quad));
           if (stay) add = __dadd_rn(add, Lps[r]);
           BC(c, D + 2 * KS) = __dadd_rn(BP(p, D + 2 * KS), add);
+          if constexpr (PATH) {
+            K3_PATH_PTRS;
+            pa.vC[c] = __dadd_rn(pa.vP[p], add);
+          }
           codeC[c] = ((codeP[p] << bits) | (unsigned long long)label(c)) & cmask;
           if (!FOLLOW && !reg_grouping) gid[c] = -1;
         }
@@ -626,6 +684,11 @@ __global__ void __launch_bounds__(32 * XT_K3_WARPS, XT_K3_MIN_CTAS) k3_predict(c
               for (int q = 0; q < CO; ++q) BP(g, q) = BC(c0, q);
               rw[c0] = 1.0;
               rg[c0] = (uint16_t)g;
+              if constexpr (PATH) {
+                K3_PATH_PTRS;
+                pa.vP[g] = pa.vC[c0];
+                pa.recArg[(size_t)step * capP + g] = (uint16_t)c0;
+              }
               if (!FOLLOW) {  // (history window and codes only serve this track's own decisions)
                 const int lab = label(c0), p0 = c0 / K;
                 for (int s = 0; s < nS; ++s) HISTN(g, 0, s) = (lab == s) ? 1.0 : 0.0;
@@ -669,6 +732,21 @@ __global__ void __launch_bounds__(32 * XT_K3_WARPS, XT_K3_MIN_CTAS) k3_predict(c
                 rw[c] = __ddiv_rn(aC[c], sw);
               }
               aP[g] = sw;  // (aP, like aC, is only used after the forward pass) for the history rows below
+              if constexpr (PATH) {  // the group's path score: its best member's (ties: the first in member order)
+                K3_PATH_PTRS;
+                double bv = pa.vC[c0];
+                int bc = c0;
+                #pragma unroll 1
+                for (int k = 1; k < n; ++k) {
+                  const int c = order[o + k];
+                  if (pa.vC[c] > bv) {
+                    bv = pa.vC[c];
+                    bc = c;
+                  }
+                }
+                pa.vP[g] = bv;
+                pa.recArg[(size_t)step * capP + g] = (uint16_t)bc;
+              }
             }
             curP[g] = c0 % nS;  // newest true state (curP / codeP are only read by the expansion)
           }
@@ -783,6 +861,13 @@ __global__ void __launch_bounds__(32 * XT_K3_WARPS, XT_K3_MIN_CTAS) k3_predict(c
           e2[D + KS + 1] = (double)(c % nS);
           continue;
         }
+        if constexpr (PATH) {  // the final path score, in place of V
+          K3_PATH_PTRS;
+          double* fv = have_children ? pa.vC : pa.vP;
+          double vs = fv[c] + term;
+          if (ck.isBL) vs += Lsm[c % nS];
+          fv[c] = vs;
+        }
         if (ck.isBL) v += Lsm[c % nS];
         aC[c] = v;
         vmax = fmax(vmax, v);
@@ -807,6 +892,42 @@ __global__ void __launch_bounds__(32 * XT_K3_WARPS, XT_K3_MIN_CTAS) k3_predict(c
       #pragma unroll 1
       for (int c = lane; c < nP; c += 32) aC[c] *= inv;
       __syncwarp();
+      if constexpr (PATH) {
+        // the best final sequence (ties: the lowest index), then the backtrack along the recorded argmax members
+        K3_PATH_PTRS;
+        const double* fv = have_children ? pa.vC : pa.vP;
+        double pbest = -INFINITY;
+        int pc = -1;
+        #pragma unroll 1
+        for (int c = lane; c < nP; c += 32) {
+          if (pc < 0 || fv[c] > pbest) {
+            pbest = fv[c];
+            pc = c;
+          }
+        }
+#pragma unroll
+        for (int o2 = 16; o2 > 0; o2 >>= 1) {
+          const double ov = __shfl_xor_sync(0xffffffffu, pbest, o2);
+          const int oc = __shfl_xor_sync(0xffffffffu, pc, o2);
+          if (oc >= 0 && (pc < 0 || ov > pbest || (ov == pbest && oc < pc))) {
+            pbest = ov;
+            pc = oc;
+          }
+        }
+        if (lane == 0) {  // the label of the chosen child at every level, then its parent's best member
+          int8_t* lab = (int8_t*)a.path[0] + (size_t)ck.loc_off + (size_t)t * L;
+          int c = pc;
+          #pragma unroll 1
+          for (int s = L - 1; s >= 2; --s) {
+            lab[s] = (int8_t)label(c);
+            const int p = c / K;
+            c = s > 2 ? (int)pa.recArg[(size_t)(s - 1) * capP + p] : p;
+          }
+          lab[1] = (int8_t)(c % nS);  // initial sequence c = h0 + nS*h1: row 1 = h0, row 0 = h1
+          lab[0] = (int8_t)(c / nS);
+          ((double*)a.path[1])[(size_t)ck.trk_off + t] = pbest - (log(ssum) + vmax);
+        }
+      }
 
       // ---- backward sweep over the recorded lattice (deterministic warp reductions) ----
       // aC holds the posterior of the sequences *after* the expansion of `step`.
@@ -893,4 +1014,5 @@ __global__ void __launch_bounds__(32 * XT_K3_WARPS, XT_K3_MIN_CTAS) k3_predict(c
 #undef HISTN
 #undef DDX
 #undef LROW
+#undef K3_PATH_PTRS
 }

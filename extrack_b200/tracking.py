@@ -727,6 +727,57 @@ def predict_residuals(all_tracks, dt, params, cell_dims=[1], nb_states=4, frame_
                      gather, "resid")
 
 
+def predict_path(all_tracks, dt, params, cell_dims=[1], nb_states=4, frame_len=5, max_nb_states=200, threshold=0.1,
+                 workers=1, input_LocErr=None, verbose=0, nb_max=1, gather=True):
+    """``predict_Bs`` plus the most probable state path (MAP / Viterbi path) of every track: ``(preds, paths,
+    path_logp)``, three ``{str(L): array}`` dictionaries.  ``preds[k]`` is ``predict_Bs``'s float64[n, L, nb_states];
+    ``paths[k]`` is int8[n, L], one state label per localisation (forward time); ``path_logp[k]`` is float64[n].
+
+    The annotation recursion is a lattice: every expansion gives each child one parent, every fusion gives each member
+    a normalised merge weight inside its group, and the final sequences get softmax(LP).  A route from an initial to a
+    final sequence weighs its final weight times the product of the merge weights along it; the route weights sum to 1,
+    and summed by label they are ``preds``.  ``paths`` is the label sequence of the heaviest route (ties: the lowest
+    member / sequence index) and ``path_logp`` the log of its weight, so ``path_logp <= log preds[t, k, paths[t, k]]``
+    for every k.  Without fusion (tracks no longer than ``frame_len``) the path is the exact most probable state
+    sequence and ``path_logp`` its posterior log-probability.  Unlike ``argmax(preds, -1)``, which maximises the
+    expected number of correct frames, the path is one consistent segmentation: it does not dither where the
+    posteriors are near 0.5.  ``path_segments`` turns the paths into dwell-time histograms.  Labels are those of
+    ``preds`` (with the reference's int8 label wrap, which only matters for 3, 5, ... states past 128 sequences).
+
+    Arguments, validation, ``nb_max`` rules and errors, ``torch.distributed`` sharding and ``gather`` are those of
+    ``predict_Bs`` (paths and path_logp take one more all-gather per bucket each).
+    """
+    return _annotate(all_tracks, dt, params, cell_dims, nb_states, frame_len, max_nb_states, threshold, input_LocErr, nb_max,
+                     gather, "path")
+
+
+def path_segments(paths, nb_states):
+    """Run lengths of the MAP segments of ``predict_path``'s paths (host only): ``(interior, censored)``, two int64
+    arrays [L_max, nb_states] (L_max: the longest bucket's length).  Row ``n - 1`` counts the segments of n
+    localisations, by state (the layout of ``xt_seglen_hist``).  ``interior`` holds the segments whose both ends are
+    observed inside the track: the dwell-time histogram to fit.  ``censored`` holds those that touch the first or the
+    last localisation of their track, whose true length is unknown (a track without a switch is one censored segment of
+    its full length)."""
+    items = [np.asarray(a) for a in (paths.values() if isinstance(paths, dict) else paths)]
+    L_max = max((a.shape[1] for a in items if a.ndim == 2), default=0)
+    interior = np.zeros((L_max, nb_states), dtype=np.int64)
+    censored = np.zeros((L_max, nb_states), dtype=np.int64)
+    for a in items:
+        if a.size == 0:
+            continue
+        a = a.astype(np.int64)
+        n, L = a.shape
+        change = a[:, 1:] != a[:, :-1]  # [n, L - 1]: a segment ends at localisation k and the next starts at k + 1
+        t_e, k_e = np.nonzero(np.concatenate([change, np.ones((n, 1), dtype=bool)], axis=1))
+        _, k_s = np.nonzero(np.concatenate([np.ones((n, 1), dtype=bool), change], axis=1))
+        # (row-major order: the i-th start and the i-th end belong to the same segment)
+        length, state = k_e - k_s + 1, a[t_e, k_e]
+        cens = (k_s == 0) | (k_e == L - 1)
+        np.add.at(interior, (length[~cens] - 1, state[~cens]), 1)
+        np.add.at(censored, (length[cens] - 1, state[cens]), 1)
+    return interior, censored
+
+
 def transition_summary(preds, pairs):
     """Switching statistics from ``predict_transitions``' outputs (host only).
 
@@ -752,8 +803,8 @@ def transition_summary(preds, pairs):
 
 def _annotate(all_tracks, dt, params, cell_dims, nb_states, frame_len, max_nb_states, threshold, input_LocErr, nb_max, gather,
               kind):
-    """Body of predict_Bs ("preds"), predict_transitions ("pairs") and predict_residuals ("resid"): the posteriors and
-    the arrays of that output kind, each as a {str(L): array} dictionary."""
+    """Body of predict_Bs ("preds"), predict_transitions ("pairs"), predict_residuals ("resid") and predict_path
+    ("path"): the posteriors and the arrays of that output kind, each as a {str(L): array} dictionary."""
     sorted_tracks, l_list = _sorted_buckets(all_tracks)
     keys = [k for k in l_list if len(all_tracks[k]) > 0]
     sorted_LocErrs = [np.asarray(input_LocErr[k], dtype=np.float64) for k in keys] if input_LocErr is not None else None
@@ -776,8 +827,11 @@ def _annotate(all_tracks, dt, params, cell_dims, nb_states, frame_len, max_nb_st
         "preds": [],
         "pairs": [lambda L: (L - 1, nb_states, nb_states)],
         "resid": [lambda L: (L,), lambda L: (L, d)],
+        "path": [lambda L: (L,), lambda L: ()],
     }[kind]
-    outs = [{l: np.empty((0,) + rs(int(l))) for l in l_list} for rs in row_shapes]
+    # the paths are int8 labels (gathered as float64, exact for labels < 2^53, and cast back)
+    dtypes = [np.int8 if (kind == "path" and i == 1) else np.float64 for i in range(len(row_shapes))]
+    outs = [{l: np.empty((0,) + rs(int(l)), dtype=dt_) for l in l_list} for rs, dt_ in zip(row_shapes, dtypes)]
     if not sorted_tracks:
         return tuple(outs)
     for a in sorted_tracks:
@@ -803,7 +857,7 @@ def _annotate(all_tracks, dt, params, cell_dims, nb_states, frame_len, max_nb_st
     cuts = [predict_shard(len(a), rank, world, nb_max) for a in sorted_tracks]
     mine = [b for b, (lo, hi) in enumerate(cuts) if hi > lo]
     loc = lambda arrs: [arrs[b][cuts[b][0]:cuts[b][1]] for b in mine] if arrs is not None else None
-    local = [[np.empty((0,) + rs(a.shape[1])) for a in sorted_tracks] for rs in row_shapes]
+    local = [[np.empty((0,) + rs(a.shape[1]), dtype=dt_) for a in sorted_tracks] for rs, dt_ in zip(row_shapes, dtypes)]
     if mine:
         eng = _native.Engine(_default_device())
         try:
@@ -821,6 +875,8 @@ def _annotate(all_tracks, dt, params, cell_dims, nb_states, frame_len, max_nb_st
                 res = eng.predict_pairs(p, nb_states)
             elif kind == "resid":
                 res = eng.predict_residuals(p, nb_states)
+            elif kind == "path":
+                res = eng.predict_path(p, nb_states)
             else:
                 res = (eng.predict(p, nb_states),)
             for lo, arrs in zip(local, res):
@@ -828,10 +884,10 @@ def _annotate(all_tracks, dt, params, cell_dims, nb_states, frame_len, max_nb_st
                     lo[b] = x
         finally:
             eng.close()
-    for out, lo, rs in zip(outs, local, row_shapes):
+    for out, lo, rs, dt_ in zip(outs, local, row_shapes, dtypes):
         full = lo if (world == 1 or not gather) else _gather_predictions(lo, sorted_tracks, world, rs, nb_max)
         for a, x in zip(sorted_tracks, full):
-            out[str(a.shape[1])] = x
+            out[str(a.shape[1])] = np.asarray(x).astype(dt_, copy=False)
     return tuple(outs)
 
 

@@ -200,6 +200,19 @@ int xt_predict_pairs(xt_ctx* ctx, const xt_params* p, double* const* out, double
 int xt_predict_residuals(xt_ctx* ctx, const xt_params* p, double* const* out, double* const* logpred, double* const* pit);
 
 /*
+ * State annotation with the most probable state path (MAP / Viterbi path): xt_predict (same options, plans and errors,
+ * same out[s]) that also fills path[s] with int8_t[n[s]][L[s]] and path_logp[s] with double[n[s]].  The recursion is a
+ * lattice: every expansion gives each child one parent, every fusion gives each member a normalised merge weight w inside
+ * its group, the final sequences get softmax(LP).  A route from an initial to a final sequence weighs its final softmax
+ * weight times the product of the w along it; the route weights sum to 1 and, summed by label, give out[s].
+ *   path[s][t][k]   = the state label at localisation k of track t's heaviest route (ties: lowest member / index)
+ *   path_logp[s][t] = log of that route's weight (<= 0, and <= log out[s][t][k][path[s][t][k]] for every k)
+ * Labels are those of out[s] (the int8 wrap included unless disabled).  Without fusion the path is the exact argmax over
+ * all state sequences and path_logp its posterior log-probability.
+ */
+int xt_predict_path(xt_ctx* ctx, const xt_params* p, double* const* out, int8_t* const* path, double* const* path_logp);
+
+/*
  * Position refinement — replaces extrack/refined_localization.py:207-338 (get_pos_PDF + the weighted means of
  * position_refinement) for the uploaded tracks.  Upload every length bucket as ONE chunk (chunk_size >= its track
  * count): the reference hands whole buckets to get_LC_Km_Ks (:48-204), whose grouping plan comes from the bucket's first
