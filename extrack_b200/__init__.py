@@ -4,7 +4,8 @@ Only the hot path of ``extrack.tracking`` is provided: ``param_fitting`` / ``cum
 ``Proba_Cs`` / ``predict_Bs`` and the parameter builders (plus ``predict_transitions`` / ``transition_summary``: the
 per-step two-state posteriors of the same annotation, and ``predict_residuals``: its one-step-ahead predictive
 densities and PIT values, and ``predict_path`` / ``path_segments``: its most probable state paths and their dwell
-times), plus the data formats either side of it:
+times), and ``param_uncertainty``: standard errors of fitted parameters from per-track scores along the frozen grouping
+plan, plus the data formats either side of it:
 ``readers.read_table`` (table -> length-bucketed ``all_tracks``) and ``simulate.sim_tracks``.  See DESIGN.md.
 """
 from . import readers, tracking  # noqa: F401
@@ -15,7 +16,9 @@ from .tracking import (  # noqa: F401
     generate_params,
     get_2DSPT_params,
     get_params,
+    ParamUncertainty,
     param_fitting,
+    param_uncertainty,
     path_segments,
     predict_Bs,
     predict_path,

@@ -85,6 +85,8 @@ EXPORTS = (
     "xt_sum_logp_host",
     "xt_sum_logp_async",
     "xt_chunk_logp",
+    "xt_eval_frozen",
+    "xt_score_outer",
     "xt_plan_dump",
     "xt_predict",
     "xt_predict_pairs",
@@ -107,6 +109,8 @@ EXPORTS = (
     "xt_multi_set_stay_tables",
     "xt_multi_sum_logp",
     "xt_multi_chunk_logp",
+    "xt_multi_eval_frozen",
+    "xt_multi_score_outer",
     "xt_multi_set_option",
     "xt_multi_device_load",
     "xt_multi_get_stats",
@@ -141,6 +145,10 @@ def load_library() -> C.CDLL:
     lib.xt_sum_logp_host.argtypes = [vp, i32, P(i32), P(i64), P(i32), P(vp), i32, i32, P(XtParams), P(dbl)]
     lib.xt_sum_logp_async.argtypes = [vp, P(XtParams), vp, vp]
     lib.xt_chunk_logp.argtypes = [vp, i32, P(XtParams), P(dbl)]
+    lib.xt_eval_frozen.argtypes = [vp, i32, P(XtParams), P(dbl), P(vp)]
+    lib.xt_score_outer.argtypes = [vp, i32, P(XtParams), P(XtParams), P(dbl), P(dbl), P(dbl), P(dbl), P(dbl)]
+    lib.xt_multi_eval_frozen.argtypes = [vp, i32, P(XtParams), P(dbl)]
+    lib.xt_multi_score_outer.argtypes = [vp, i32, P(XtParams), P(XtParams), P(dbl), P(dbl), P(dbl), P(dbl), P(dbl)]
     lib.xt_plan_dump.argtypes = [vp, i32, i32, P(i32), P(i32), P(i32), i32, P(dbl)]
     lib.xt_predict.argtypes = [vp, P(XtParams), P(vp)]
     lib.xt_predict_pairs.argtypes = [vp, P(XtParams), P(vp), P(vp)]
@@ -189,6 +197,30 @@ def _raise(code: int, msg: str):
     if code == XT_ERR_UNSUPPORTED:
         raise NotImplementedError(msg)
     raise EngineError(code, msg)
+
+
+XT_MAX_SCORE_DIRS = 32
+
+
+def _param_array(ps: Sequence[XtParams]):
+    arr = (XtParams * len(ps))()
+    for k, p in enumerate(ps):
+        arr[k] = p
+    return arr
+
+
+def _score_outer(fn, h, p_plus: Sequence[XtParams], p_minus: Sequence[XtParams], inv_2h) -> dict:
+    """Shared body of Engine.score_outer / MultiEngine.score_outer (``fn`` = the C entry point)."""
+    n = len(p_plus)
+    if len(p_minus) != n or len(inv_2h) != n:
+        raise ValueError("score_outer: p_plus, p_minus and inv_2h need the same length")
+    dp = C.POINTER(C.c_double)
+    inv = np.ascontiguousarray(inv_2h, dtype=np.float64)
+    sp, sm, gs = np.empty(n), np.empty(n), np.empty(n)
+    gram = np.empty((n, n))
+    rc = fn(h, n, _param_array(p_plus), _param_array(p_minus), inv.ctypes.data_as(dp), sp.ctypes.data_as(dp),
+            sm.ctypes.data_as(dp), gs.ctypes.data_as(dp), gram.ctypes.data_as(dp))
+    return rc, {"sum_plus": sp, "sum_minus": sm, "gsum": gs, "gram": gram}
 
 
 class Engine:
@@ -315,6 +347,24 @@ class Engine:
     def chunk_logp(self, chunk: int, nT: int, p: XtParams) -> np.ndarray:
         out = np.empty(nT, dtype=np.float64)
         self._check(self._lib.xt_chunk_logp(self._h, int(chunk), C.byref(p), out.ctypes.data_as(C.POINTER(C.c_double))))
+        return out
+
+    def eval_frozen(self, ps: Sequence[XtParams], per_track: bool = False):
+        """Sums of log P for every parameter set along the resident plan (``xt_eval_frozen``); with ``per_track`` also
+        float64[len(ps), n_tracks] per-track values in upload order.  Returns ``sums`` or ``(sums, per_track)``."""
+        sums = np.empty(len(ps))
+        n_tracks = sum(n for (_, n) in self.segments)
+        lps = np.empty((len(ps), n_tracks)) if per_track else None
+        ptrs = (C.c_void_p * len(ps))(*[r.ctypes.data for r in lps]) if per_track else None
+        self._check(self._lib.xt_eval_frozen(self._h, len(ps), _param_array(ps), sums.ctypes.data_as(C.POINTER(C.c_double)),
+                                             ptrs))
+        return (sums, lps) if per_track else sums
+
+    def score_outer(self, p_plus: Sequence[XtParams], p_minus: Sequence[XtParams], inv_2h) -> dict:
+        """Central-difference scores along the resident plan (``xt_score_outer``): dict of ``sum_plus``, ``sum_minus``,
+        ``gsum`` [n] and ``gram`` [n, n]."""
+        rc, out = _score_outer(self._lib.xt_score_outer, self._h, p_plus, p_minus, inv_2h)
+        self._check(rc)
         return out
 
     def plan_dump(self, chunk: int, step: int, cap: int = 4096):
@@ -512,6 +562,18 @@ class MultiEngine:
     def chunk_logp(self, chunk: int, nT: int, p: XtParams) -> np.ndarray:
         out = np.empty(nT, dtype=np.float64)
         self._check(self._lib.xt_multi_chunk_logp(self._h, int(chunk), C.byref(p), out.ctypes.data_as(C.POINTER(C.c_double))))
+        return out
+
+    def eval_frozen(self, ps: Sequence[XtParams]) -> np.ndarray:
+        """Sums of log P along every device's resident plan (``xt_multi_eval_frozen``), global chunk order."""
+        sums = np.empty(len(ps))
+        self._check(self._lib.xt_multi_eval_frozen(self._h, len(ps), _param_array(ps), sums.ctypes.data_as(C.POINTER(C.c_double))))
+        return sums
+
+    def score_outer(self, p_plus: Sequence[XtParams], p_minus: Sequence[XtParams], inv_2h) -> dict:
+        """``xt_multi_score_outer``: same result, with the same bits, as one context holding all chunks."""
+        rc, out = _score_outer(self._lib.xt_multi_score_outer, self._h, p_plus, p_minus, inv_2h)
+        self._check(rc)
         return out
 
     def set_option(self, name: str, value: int):

@@ -149,6 +149,21 @@ struct xt_ctx {
   double* d_stay[2] = {nullptr, nullptr};   // [0] per chunk, [1] per track: Lp_stay [rows][K]
   double* d_leave[2] = {nullptr, nullptr};  // [0] per chunk: linear sums [rows][nS]; [1] per track: log-sums [rows][nS]
   int stay_K[2] = {0, 0}, stay_H[2] = {0, 0};
+  // frozen evaluations (xt_eval_frozen / xt_score_outer): the replay launch of the last evaluation, repeated with other
+  // parameters along its plan.  Outputs go to buffers of their own, so the state above is never touched.
+  int frozen_kind = 0;          // 0: no plan resident; XT_FROZEN_FUSED / XT_FROZEN_OLD: the replay kernel that plan's evaluation ran
+  int frozen_Pcap = 0;          // parent slots that launch was sized with (>= max_nP of every chunk summary)
+  xt_params frozen_sig{};       // the parameters of that evaluation (structure check)
+  double* d_flogp = nullptr;    // [slots][n_tracks] per-track log P
+  size_t flogp_elems = 0;
+  double* d_fpartial = nullptr; // per-tile partial sums
+  double* d_fcsum = nullptr;    // [n_eval][n_chunks] chunk sums, and its pinned mirror
+  double* h_fcsum = nullptr;
+  size_t fcsum_elems = 0;
+  double* d_fgram = nullptr;    // [n_chunks][E] score / outer-product partials of k_score_gram, and its pinned mirror
+  double* h_fgram = nullptr;
+  size_t fgram_elems = 0;
+  int* d_fspec = nullptr;       // speculation word of the frozen launches (never set: their sizes come from the summaries)
 };
 
 static std::string g_create_error;
@@ -208,6 +223,7 @@ static void free_plan(xt_ctx* ctx) {
   ctx->plan = XtPlanPtrs{};
   ctx->d_state1 = ctx->d_hist1 = nullptr;
   ctx->cap = 0;
+  ctx->frozen_kind = 0;
 }
 
 static void free_data(xt_ctx* ctx) {
@@ -228,6 +244,12 @@ static void free_data(xt_ctx* ctx) {
   cudaFree(ctx->d_redo);
   ctx->d_redo = nullptr;
   ctx->plan_valid = false;
+  cudaFree(ctx->d_flogp); cudaFree(ctx->d_fpartial); cudaFree(ctx->d_fcsum); cudaFree(ctx->d_fgram); cudaFree(ctx->d_fspec);
+  if (ctx->h_fcsum) cudaFreeHost(ctx->h_fcsum);
+  if (ctx->h_fgram) cudaFreeHost(ctx->h_fgram);
+  ctx->d_flogp = ctx->d_fpartial = ctx->d_fcsum = ctx->h_fcsum = ctx->d_fgram = ctx->h_fgram = nullptr;
+  ctx->d_fspec = nullptr;
+  ctx->flogp_elems = ctx->fcsum_elems = ctx->fgram_elems = 0;
   cudaFree(ctx->d_tail);
   if (ctx->h_tail) cudaFreeHost(ctx->h_tail);
   ctx->d_tail = ctx->h_tail = nullptr;
@@ -487,6 +509,7 @@ static int setup_layout(xt_ctx* ctx, int32_t n_seg, const int32_t* L, const int6
   }
   ctx->have_eval = false;
   ctx->plan_valid = false;  // new coordinates: the resident plan describes the previous data set
+  ctx->frozen_kind = 0;
   // two staging buffers (AoS as on the host) overlap the copy of one segment with the repack of another
   if ((size_t)max_seg_elems > ctx->stage_elems) {
     for (int b = 0; b < 2; ++b) {
@@ -589,6 +612,7 @@ extern "C" int xt_upload_aux(xt_ctx* ctx, int32_t k_sigma, const double* const* 
   ctx->aux_has_dt = dt ? 1 : 0;
   ctx->have_eval = false;
   ctx->plan_valid = false;
+  ctx->frozen_kind = 0;
   const int chunk_size = (int)ctx->upload_sig[2];
   int slot = 0;
   for (int pass = 0; pass < 2; ++pass) {
@@ -625,6 +649,7 @@ extern "C" int xt_set_stay_tables(xt_ctx* ctx, int32_t per_track, int32_t K, int
   ctx->stay_K[i] = ctx->stay_H[i] = 0;
   ctx->have_eval = false;
   ctx->plan_valid = false;
+  ctx->frozen_kind = 0;  // (per-chunk tables are context state the frozen launches would read)
   if (!Lp_stay || !L_leave) return XT_OK;
   if (ctx->chunks.empty() || K < 1 || H < K || H % K != 0) {
     set_error(ctx, "xt_set_stay_tables: upload the tracks first; need K >= 1 and H a multiple of K");
@@ -1130,6 +1155,14 @@ static void mark_plan_valid(xt_ctx* ctx, const xt_params* p) {
   ctx->plan_valid = true;
   ctx->plan_sig = *p;
 }
+#define XT_FROZEN_FUSED 1  // fused replay kernel (shared- or global-memory state, VAR instantiation included)
+#define XT_FROZEN_OLD 2    // first-generation linear-domain / log-domain kernel of the two-phase path
+// the evaluation that just succeeded left a plan for the frozen entry points: which replay launch it ran
+static void mark_frozen(xt_ctx* ctx, const xt_params* p, int kind, int Pcap) {
+  ctx->frozen_kind = kind;
+  ctx->frozen_Pcap = Pcap;
+  ctx->frozen_sig = *p;
+}
 
 #define XT_RETRY 1        // internal: the speculative single-pass evaluation has to be redone in two phases
 #define XT_RETRY_EARLY 2  // same, and nothing was enqueued yet (host buffers not copied)
@@ -1239,6 +1272,7 @@ static int evaluate_pipelined(xt_ctx* ctx, const xt_params* p, int bits, double*
   ctx->have_eval = true;
   ctx->last_fused = true;
   mark_plan_valid(ctx, p);
+  mark_frozen(ctx, p, XT_FROZEN_FUSED, fl.fa.Pcap);
   return XT_OK;
 }
 
@@ -1381,6 +1415,57 @@ static int evaluate_verified(xt_ctx* ctx, const xt_params* p, int bits, double* 
   ctx->last_p = *p;
   ctx->have_eval = true;
   mark_plan_valid(ctx, p);
+  mark_frozen(ctx, p, XT_FROZEN_FUSED, fl.fa.Pcap);
+  return XT_OK;
+}
+
+// first-generation linear-domain replay kernel (k2_variant 1) or its log-domain global-memory variant, over all chunks
+// with Pmax parent slots; per-track log P to `logp`, per-tile partial sums to `partial` (plain work table)
+static int enqueue_old(xt_ctx* ctx, const xt_params* p, int Pmax, double* logp, double* partial) {
+  const int K = ipow(p->nS, p->nsub);
+  const int KS = p->n_loc, CO = p->d + KS + 1;
+  K2Args a{};
+  a.chunks = ctx->d_chunks;
+  a.work = ctx->d_work;
+  a.soa = ctx->d_soa;
+  a.plan = ctx->plan;
+  a.summ = ctx->d_summ;
+  a.logp = logp;
+  a.partial = partial;
+  a.Pcap = Pmax;
+  a.n_work = (int)ctx->work.size();
+  leave_sums(p, a.Lsum);
+  K2Lin lin{};
+  for (int h = 0; h < K * p->nS; ++h) {
+    lin.winit[h] = std::exp(p->LT[h] + p->LF[h]);
+    lin.tau0[h] = std::exp(p->LT[h]);
+    lin.tau1[h] = std::exp(p->LT[h] + p->Lp_stay[h % K]);
+  }
+  for (int s = 0; s < p->nS; ++s) lin.leave[s] = std::exp(a.Lsum[s]);
+  const int wpc = ctx->k2_wpc;
+  const size_t state_bytes = (size_t)2 * Pmax * CO * 32 * sizeof(double);
+  const size_t smem = state_bytes + (size_t)2 * wpc * 32 * sizeof(double);
+  const bool use_smem = smem <= (size_t)ctx->smem_optin && !ctx->force_global && !is_var(p);
+  if (is_var(p)) {
+    a.ax = make_aux(ctx, p, 0);
+    if (p->flags & XT_FLAG_VAR_DT) dd_unit(p, a.ddu);
+  }
+  int grid = a.n_work;
+  if (!use_smem) {
+    grid = std::min(a.n_work, ctx->n_sm * ctx->k2_global_ctas);
+    const size_t need = (size_t)grid * state_bytes;
+    if (need > ctx->gstate_bytes) {
+      cudaFree(ctx->d_gstate);
+      ctx->d_gstate = nullptr;
+      ctx->gstate_bytes = 0;
+      XT_CUDA_OK(cudaMalloc(&ctx->d_gstate, need));
+      ctx->gstate_bytes = need;
+    }
+    a.gstate = ctx->d_gstate;
+  }
+  const cudaError_t e = xt_launch_k2_old(a, *p, lin, smem, use_smem, grid, wpc, ctx->stream);
+  XT_CUDA_OK(e);
+  ctx->stats.k2_launches++;
   return XT_OK;
 }
 
@@ -1396,6 +1481,7 @@ static int evaluate(xt_ctx* ctx, const xt_params* p, double* d_out, const double
   XT_CUDA_OK(cudaSetDevice(ctx->device));
   ctx->stats = xt_stats{};
   ctx->csum_fetched = false;
+  ctx->frozen_kind = 0;  // (set again when this evaluation succeeds)
   if (!xyz && ctx->pipeline && ctx->plan_verify && ctx->plan_valid && ctx->last_fused && same_structure(*p, ctx->plan_sig)) {
     rc = evaluate_verified(ctx, p, bits, d_out);
     if (rc != XT_RETRY && rc != XT_RETRY_EARLY) return rc;
@@ -1432,7 +1518,10 @@ static int evaluate(xt_ctx* ctx, const xt_params* p, double* d_out, const double
     if (rc) return rc;
     ctx->last_fused = true;
     rc = finish_eval(ctx, p, fl.tpt - 1, d_out, su, sg, maxC);
-    if (rc == XT_OK) mark_plan_valid(ctx, p);
+    if (rc == XT_OK) {
+      mark_plan_valid(ctx, p);
+      mark_frozen(ctx, p, XT_FROZEN_FUSED, Pmax);
+    }
     return rc;
   }
   if (ctx->last_fused || !ctx->plan_has_grec) {  // the plan was written without the records this path reads
@@ -1441,51 +1530,11 @@ static int evaluate(xt_ctx* ctx, const xt_params* p, double* d_out, const double
     if (rc) return rc;
   }
   // first-generation linear-domain kernel (k2_variant 1) or log-domain global-memory fallback
-  const int K = ipow(p->nS, p->nsub);
-  const int KS = p->n_loc, CO = p->d + KS + 1;
-  K2Args a{};
-  a.chunks = ctx->d_chunks;
-  a.work = ctx->d_work;
-  a.soa = ctx->d_soa;
-  a.plan = ctx->plan;
-  a.summ = ctx->d_summ;
-  a.logp = ctx->d_logp;
-  a.partial = ctx->d_partial;
-  a.Pcap = Pmax;
-  a.n_work = (int)ctx->work.size();
-  leave_sums(p, a.Lsum);
-  K2Lin lin{};
-  for (int h = 0; h < K * p->nS; ++h) {
-    lin.winit[h] = std::exp(p->LT[h] + p->LF[h]);
-    lin.tau0[h] = std::exp(p->LT[h]);
-    lin.tau1[h] = std::exp(p->LT[h] + p->Lp_stay[h % K]);
-  }
-  for (int s = 0; s < p->nS; ++s) lin.leave[s] = std::exp(a.Lsum[s]);
-  const int wpc = ctx->k2_wpc;
-  const size_t state_bytes = (size_t)2 * Pmax * CO * 32 * sizeof(double);
-  const size_t smem = state_bytes + (size_t)2 * wpc * 32 * sizeof(double);
-  const bool use_smem = smem <= (size_t)ctx->smem_optin && !ctx->force_global && !is_var(p);
-  if (is_var(p)) {
-    a.ax = make_aux(ctx, p, 0);
-    if (p->flags & XT_FLAG_VAR_DT) dd_unit(p, a.ddu);
-  }
-  int grid = a.n_work;
-  if (!use_smem) {
-    grid = std::min(a.n_work, ctx->n_sm * ctx->k2_global_ctas);
-    const size_t need = (size_t)grid * state_bytes;
-    if (need > ctx->gstate_bytes) {
-      cudaFree(ctx->d_gstate);
-      ctx->d_gstate = nullptr;
-      ctx->gstate_bytes = 0;
-      XT_CUDA_OK(cudaMalloc(&ctx->d_gstate, need));
-      ctx->gstate_bytes = need;
-    }
-    a.gstate = ctx->d_gstate;
-  }
-  const cudaError_t e = xt_launch_k2_old(a, *p, lin, smem, use_smem, grid, wpc, ctx->stream);
-  XT_CUDA_OK(e);
-  ctx->stats.k2_launches++;
-  return finish_eval(ctx, p, 2, d_out, su, sg, maxC);
+  rc = enqueue_old(ctx, p, Pmax, ctx->d_logp, ctx->d_partial);
+  if (rc) return rc;
+  rc = finish_eval(ctx, p, 2, d_out, su, sg, maxC);
+  if (rc == XT_OK) mark_frozen(ctx, p, XT_FROZEN_OLD, Pmax);
+  return rc;
 }
 
 extern "C" int xt_sum_logp(xt_ctx* ctx, const xt_params* p, double* out) {
@@ -1520,6 +1569,7 @@ extern "C" int xt_sum_logp_async(xt_ctx* ctx, const xt_params* p, double* d_out,
 extern "C" int xt_set_option(xt_ctx* ctx, const char* name, int value) {
   if (!ctx || !name) return XT_ERR_ARG;
   ctx->plan_valid = false;  // (records and schedules depend on the options: the next evaluation plans from scratch)
+  ctx->frozen_kind = 0;
   if (std::strcmp(name, "plan_verify") == 0) {
     ctx->plan_verify = value != 0;
     return XT_OK;
@@ -1763,3 +1813,4 @@ extern "C" int xt_fp64_peak_tflops(xt_ctx* ctx, double* out) {
 #include "xt_refine_host.inl"
 #include "xt_seglen_host.inl"
 #include "xt_multi.inl"
+#include "xt_frozen_host.inl"

@@ -15,6 +15,7 @@ distinct list of arrays handed to ``cum_Proba_Cs``) and stay resident on the GPU
 from __future__ import annotations
 
 import ctypes
+from dataclasses import dataclass
 from typing import Dict, List, Optional, Sequence
 
 import numpy as np
@@ -453,6 +454,48 @@ class TrackSet:
             raise _native.EngineError(_native.XT_ERR_STATE, "the likelihood evaluation failed on another rank")
         return total
 
+    def _all_reduce(self, compute, size: int) -> np.ndarray:
+        """``compute()`` -> float64[size] on this rank's shard, summed over the ranks in one all-reduce that also carries
+        the error flag (as ``sum_logp``)."""
+        if self.world_size == 1:
+            return compute()
+        import torch
+        import torch.distributed as dist
+
+        dev = torch.device("cuda", self.device) if dist.get_backend() == "nccl" else torch.device("cpu")
+        buf = torch.zeros(size + 1, dtype=torch.float64, device=dev)
+        err = None
+        try:
+            if self.n_local_chunks:
+                buf[:size] = torch.from_numpy(np.ascontiguousarray(compute(), dtype=np.float64)).to(dev)
+        except Exception as e:  # noqa: BLE001 - re-raised below on every rank
+            err = e
+            buf.zero_()
+            buf[size] = 1.0
+        dist.all_reduce(buf, op=dist.ReduceOp.SUM)
+        out = buf.cpu().numpy()
+        if err is not None:
+            raise err
+        if out[size] != 0.0:
+            raise _native.EngineError(_native.XT_ERR_STATE, "the frozen-plan evaluation failed on another rank")
+        return out[:size]
+
+    def eval_frozen(self, ps: Sequence[_native.XtParams]) -> np.ndarray:
+        """Sums of log P over the data set for every parameter set, along the plan of the last ``sum_logp``."""
+        return self._all_reduce(lambda: self.engine.eval_frozen(ps), len(ps))
+
+    def score_outer(self, p_plus: Sequence[_native.XtParams], p_minus: Sequence[_native.XtParams], inv_2h) -> dict:
+        """Central-difference scores along the plan of the last ``sum_logp``: ``sum_plus``, ``sum_minus``, ``gsum``,
+        ``gram`` (see ``xt_score_outer``)."""
+        n = len(p_plus)
+
+        def compute():
+            r = self.engine.score_outer(p_plus, p_minus, inv_2h)
+            return np.concatenate([r["sum_plus"], r["sum_minus"], r["gsum"], r["gram"].reshape(-1)])
+
+        v = self._all_reduce(compute, 3 * n + n * n)
+        return {"sum_plus": v[:n], "sum_minus": v[n:2 * n], "gsum": v[2 * n:3 * n], "gram": v[3 * n:].reshape(n, n)}
+
     def close(self):
         self.engine.close()
 
@@ -577,6 +620,24 @@ def invalidate_cache() -> None:
 # --------------------------------------------------------------------------------------
 # objective (tracking.py:991-1088)
 # --------------------------------------------------------------------------------------
+def _objective_tables(params, ts: TrackSet, dt, cell_dims, nb_substeps, frame_len, threshold, max_nb_states, Matrix_type):
+    """Parameters -> the objective's validity guard -> ``build_tables``: ``(p, (Ds, TrMat, pBL))``, ``p`` = None when
+    the guard rejects the parameters (the objective is then +inf)."""
+    loc, Ds, Fs, TrMat, pBL = _extract_scalars(params, nb_substeps, Matrix_type)
+    if type(dt) == list:
+        ds = _median_ds(Ds, ts.dt_mid0)[0]  # avg_ds = np.median(ds[0], axis=(0, 1)), tracking.py:1012-1013
+    else:
+        ds = np.sqrt(2 * Ds * dt)
+    # validity guard of the reference (tracking.py:1017: all transition probabilities and fractions positive, diffusion
+    # lengths ascending); minima instead of three np.all passes - NaN fails either way
+    if not (TrMat.min() > 0 and Fs.min() > 0 and (len(ds) < 2 or (ds[1:] - ds[:-1]).min() >= 0)):
+        return None, (Ds, TrMat, pBL)
+    slope = (params["slope_LocErr"].value, params["offset_LocErr"].value) if (ts.loc_k and _has_slope(params)) else None
+    p = build_tables(loc, ds, Fs, TrMat, pBL, cell_dims, nb_substeps, frame_len, ts.min_len, threshold,
+                     max_nb_states, ts.nb_dims, var_loc_k=ts.loc_k, var_dt=ts.has_dt, Ds=Ds, slope_offset=slope)
+    return p, (Ds, TrMat, pBL)
+
+
 def cum_Proba_Cs(params, all_tracks, dt, cell_dims, input_LocErr, nb_states, nb_substeps, frame_len, verbose=1,
                  workers=1, Matrix_type=1, threshold=0.2, max_nb_states=120, max_number_of_tracks_per_matrix=2000,
                  _trackset: Optional[TrackSet] = None):
@@ -587,21 +648,13 @@ def cum_Proba_Cs(params, all_tracks, dt, cell_dims, input_LocErr, nb_states, nb_
     ``dt`` a float or the matching list of ``[n, L]`` time steps (tracking.py:1024-1044).
     ``workers`` > 1 asks for that many GPUs of this box (``resolve_devices``); the GPUs replace the process pool.
     """
-    loc, Ds, Fs, TrMat, pBL = _extract_scalars(params, nb_substeps, Matrix_type)
     dt_list = dt if type(dt) == list else None
     ts = _trackset if _trackset is not None else _trackset_for(all_tracks, max_number_of_tracks_per_matrix, input_LocErr,
                                                                dt_list, workers)
     quiet = ts.rank != 0
-    if dt_list is not None:
-        ds = _median_ds(Ds, ts.dt_mid0)[0]  # avg_ds = np.median(ds[0], axis=(0, 1)), tracking.py:1012-1013
-    else:
-        ds = np.sqrt(2 * Ds * dt)
-    # validity guard of the reference (tracking.py:1017: all transition probabilities and fractions positive, diffusion
-    # lengths ascending); minima instead of three np.all passes - NaN fails either way
-    if TrMat.min() > 0 and Fs.min() > 0 and (len(ds) < 2 or (ds[1:] - ds[:-1]).min() >= 0):
-        slope = (params["slope_LocErr"].value, params["offset_LocErr"].value) if (ts.loc_k and _has_slope(params)) else None
-        p = build_tables(loc, ds, Fs, TrMat, pBL, cell_dims, nb_substeps, frame_len, ts.min_len, threshold,
-                         max_nb_states, ts.nb_dims, var_loc_k=ts.loc_k, var_dt=ts.has_dt, Ds=Ds, slope_offset=slope)
+    p, (Ds, TrMat, pBL) = _objective_tables(params, ts, dt, cell_dims, nb_substeps, frame_len, threshold, max_nb_states,
+                                            Matrix_type)
+    if p is not None:
         if ts.has_dt and ts.n_local_chunks:
             ts.engine.set_stay_tables(False, *stay_tables(Ds, ts.dt_mids, TrMat, pBL, cell_dims, nb_substeps))
         ts._last_p = p
@@ -1024,3 +1077,196 @@ def get_2DSPT_params(all_tracks, dt, nb_substeps=1, nb_states=2, frame_len=8, ve
     params = get_params(nb_states, steady_state, vary_params, estimated_vals, min_values, max_values)
     return param_fitting(all_tracks, dt, params=params, nb_states=nb_states, nb_substeps=nb_substeps, frame_len=frame_len,
                          verbose=verbose, workers=workers, method=method, steady_state=steady_state, cell_dims=cell_dims)
+
+
+# --------------------------------------------------------------------------------------
+# standard errors of fitted parameters (frozen-plan scores and observed information)
+# --------------------------------------------------------------------------------------
+@dataclass
+class ParamUncertainty:
+    """Result of ``param_uncertainty``.  Matrices are over ``names`` (free parameters with a usable step), in order.
+
+    ``hessian``: observed information H (Hessian of -log L); ``opg``: J = sum over tracks of g g^T (per-track scores g);
+    ``gradient``: sum of g (gradient of log L); ``newton_decrement``: g^T H^-1 g (near 0 at a converged fit);
+    ``covar`` = H^-1, ``covar_robust`` = H^-1 J H^-1 (sandwich, valid under misspecification); ``stderr`` /
+    ``stderr_robust``: per parameter name (NaN for ``at_bound``, None for ``vary=False``; ``expr`` parameters by the
+    delta method); ``correl``: correlation matrix of ``covar``; ``params``: a copy with ``.stderr`` / ``.correl`` set."""
+
+    names: List[str]
+    at_bound: List[str]
+    hessian: np.ndarray
+    opg: np.ndarray
+    gradient: np.ndarray
+    newton_decrement: float
+    covar: np.ndarray
+    covar_robust: np.ndarray
+    stderr: Dict[str, Optional[float]]
+    stderr_robust: Dict[str, Optional[float]]
+    correl: np.ndarray
+    params: object
+    n_evaluations: int = 0
+
+
+class InvalidPoint(Exception):
+    """Raised by an uncertainty backend when parameter list entry ``index`` fails the objective's validity guard."""
+
+    def __init__(self, index: int):
+        super().__init__(index)
+        self.index = index
+
+
+def uncertainty_from_backend(params, totals, score_outer, rel_step: float = 1e-4) -> ParamUncertainty:
+    """Standard errors by central differences of a smooth log-likelihood surface, given by two callables:
+
+    * ``totals(thetas)`` -> float64[len(thetas)]: sum of log P at every free-parameter vector;
+    * ``score_outer(th_plus, th_minus, inv_2h)`` -> dict ``sum_plus``, ``sum_minus``, ``gsum``, ``gram`` (see
+      ``xt_score_outer``).
+
+    Either may raise ``InvalidPoint(index)``.  Vectors are over the free parameters with a usable step (``names``).
+    The engine along a frozen plan is the production backend; tests drive this with oracles and synthetic surfaces."""
+    import warnings
+
+    names_all = list(params.keys())
+    free = [n for n in names_all if params[n].vary and params[n].expr is None]
+    act, held, h = [], [], []
+    for n in free:
+        if _held(params[n], rel_step):
+            held.append(n)
+        else:
+            act.append(n)
+            h.append(rel_step * abs(float(params[n].value)))
+    m = len(act)
+    if m > _native.XT_MAX_SCORE_DIRS:
+        raise ValueError("param_uncertainty: at most %d free parameters" % _native.XT_MAX_SCORE_DIRS)
+    h = np.array(h, dtype=float)
+    theta = np.array([float(params[n].value) for n in act])
+    E = np.eye(m) * h[:, None] if m else np.zeros((0, 0))
+
+    def run(fn, describe, *args):
+        try:
+            return fn(*args)
+        except InvalidPoint as e:
+            raise ValueError("param_uncertainty: the step of %s leaves the region the objective accepts (the "
+                             "parameter guard rejects the perturbed point)" % describe(e.index)) from None
+
+    plus, minus = [theta + E[i] for i in range(m)], [theta - E[i] for i in range(m)]
+    sc = run(score_outer, lambda k: act[k % m], plus, minus, 1.0 / (2.0 * h)) if m else None
+    pts, who = [theta], [None]
+    for i in range(m):
+        for j in range(i + 1, m):
+            for si, sj in ((1, 1), (1, -1), (-1, 1), (-1, -1)):
+                pts.append(theta + si * E[i] + sj * E[j])
+                who.append((i, j))
+    S = run(totals, lambda k: "%s / %s" % (act[who[k][0]], act[who[k][1]]) if who[k] else "the estimate", pts)
+    S0 = S[0]
+    H = np.zeros((m, m))
+    k = 1
+    for i in range(m):
+        H[i, i] = -(sc["sum_plus"][i] - 2.0 * S0 + sc["sum_minus"][i]) / (h[i] * h[i])
+        for j in range(i + 1, m):
+            spp, spm, smp, smm = S[k:k + 4]
+            H[i, j] = H[j, i] = -(spp - spm - smp + smm) / (4.0 * h[i] * h[j])
+            k += 4
+    J = np.array(sc["gram"], dtype=float) if m else np.zeros((0, 0))
+    g = np.array(sc["gsum"], dtype=float) if m else np.zeros(0)
+    try:
+        np.linalg.cholesky(H)
+        cov = np.linalg.inv(H)
+        cov = (cov + cov.T) / 2
+        newton = float(g @ cov @ g)
+    except np.linalg.LinAlgError:
+        warnings.warn("param_uncertainty: the observed information is not positive definite (not at a maximum, or "
+                      "a parameter is not identified); covariances are NaN", RuntimeWarning, stacklevel=2)
+        cov = np.full((m, m), np.nan)
+        newton = float("nan")
+    rob = cov @ J @ cov
+    out_params = params.copy()
+
+    def delta(C):
+        """stderr of every parameter from the covariance C of ``act``; expr parameters by the delta method."""
+        se: Dict[str, Optional[float]] = {}
+        for n in names_all:
+            p = params[n]
+            if n in act:
+                se[n] = float(np.sqrt(C[act.index(n), act.index(n)]))
+            elif n in held:
+                se[n] = float("nan")
+            elif p.expr is None:
+                se[n] = None
+            else:
+                jac = np.zeros(m)
+                for i, a in enumerate(act):  # numerical Jacobian of the expression (held parameters stay fixed)
+                    q = params.copy()
+                    q[a].value = theta[i] + h[i]
+                    vp = float(q[n].value)
+                    q[a].value = theta[i] - h[i]
+                    jac[i] = (vp - float(q[n].value)) / (2.0 * h[i])
+                se[n] = float(np.sqrt(jac @ C @ jac))
+        return se
+
+    se, se_r = delta(cov), delta(rob)
+    sd = np.sqrt(np.diag(cov))
+    correl = cov / np.outer(sd, sd) if m else np.zeros((0, 0))
+    for n in names_all:
+        out_params[n].stderr = se[n]
+        if n in act:
+            i = act.index(n)
+            out_params[n].correl = {b: float(correl[i, j]) for j, b in enumerate(act) if j != i}
+    return ParamUncertainty(act, held, H, J, g, newton, cov, rob, se, se_r, correl, out_params, 1 + 2 * m + len(pts))
+
+
+def param_uncertainty(all_tracks, dt, params, nb_states=2, nb_substeps=1, frame_len=6, workers=1, Matrix_type=1,
+                      cell_dims=[1], input_LocErr=None, threshold=0.2, max_nb_states=120, rel_step=1e-4) -> ParamUncertainty:
+    """Standard errors of fitted parameters (``params`` = ``fit.params`` or the ``param_fitting`` result itself).
+
+    Takes ``param_fitting``'s data arguments.  The objective is evaluated once at the estimate to build the grouping
+    plan; everything else runs along that frozen plan, where log P of every track is a smooth function of the
+    parameters.  Central differences (step ``rel_step * |value|``) give per-track scores and the observed information;
+    see ``ParamUncertainty`` and DESIGN.md §9.  A parameter whose value is 0, or within two steps of a bound, is held
+    fixed (listed in ``at_bound``, stderr NaN).  A ``dt`` dictionary is not supported: its field-of-view tables depend
+    on D and are per-chunk state of the engine."""
+    params = getattr(params, "params", params)
+    if isinstance(params, dict) and not hasattr(params, "valuesdict"):
+        raise TypeError("params must be lmfit Parameters or a fit result")
+    if type(dt) in (dict, list):
+        raise NotImplementedError("param_uncertainty: per-localisation dt (a dt dictionary) is not supported: the "
+                                  "field-of-view tables it needs depend on D and are per-chunk engine state")
+    sorted_tracks, l_list = _sorted_buckets(all_tracks)
+    if len(sorted_tracks) < 1:
+        raise ValueError("No track could be detected. The loaded tracks seem empty. Errors often come from wrong input paths.")
+    keys = [k for k in l_list if len(all_tracks[k]) > 0]
+    if input_LocErr is not None:
+        input_LocErr = [np.asarray(input_LocErr[k], dtype=np.float64) for k in keys]
+    ts = TrackSet([np.asarray(a, dtype=np.float64) for a in sorted_tracks], MAX_TRACKS_PER_CHUNK,
+                  input_LocErr=input_LocErr, precision="fp64", devices=resolve_devices(workers))
+    try:
+        # the free parameters the assembly steps (same rule, _held) name the entries of its vectors
+        act = [n for n in params.keys() if params[n].vary and params[n].expr is None and not _held(params[n], rel_step)]
+
+        def tables(thetas):
+            out = []
+            for k, th in enumerate(thetas):
+                q = params.copy()
+                for n, v in zip(act, th):
+                    q[n].value = float(v)
+                p, _ = _objective_tables(q, ts, dt, cell_dims, nb_substeps, frame_len, threshold, max_nb_states, Matrix_type)
+                if p is None:
+                    raise InvalidPoint(k)
+                out.append(p)
+            return out
+
+        p_hat, _ = _objective_tables(params, ts, dt, cell_dims, nb_substeps, frame_len, threshold, max_nb_states, Matrix_type)
+        if p_hat is None:
+            raise ValueError("param_uncertainty: the parameters fail the objective's validity guard")
+        ts.sum_logp(p_hat)  # the grouping plan at the estimate (every later evaluation runs along it)
+        totals = lambda thetas: ts.eval_frozen(tables(thetas))
+        score = lambda plus, minus, inv_2h: ts.score_outer(tables(plus), tables(minus), inv_2h)
+        return uncertainty_from_backend(params, totals, score, rel_step)
+    finally:
+        ts.close()
+
+
+def _held(p, rel_step) -> bool:
+    v = float(p.value)
+    step = rel_step * abs(v)
+    return v == 0.0 or v - 2 * step < p.min or v + 2 * step > p.max

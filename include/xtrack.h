@@ -25,6 +25,7 @@ extern "C" {
 #define XT_MAX_HEADS 128 /* nS^(nb_substeps+1) */
 #define XT_MAX_STATES 8
 #define XT_MAX_DIMS 3
+#define XT_MAX_SCORE_DIRS 32 /* directions of one xt_score_outer call */
 
 #define XT_OK 0
 #define XT_ERR_CUDA (-1)      /* CUDA runtime failure */
@@ -158,6 +159,35 @@ int xt_sum_logp_host(xt_ctx* ctx, int32_t n_segments, const int32_t* L, const in
  * of the previous call, which still reads or writes d_out), and `cuda_stream` is made to wait for the
  * result, so a collective can be chained without a host round trip. */
 int xt_sum_logp_async(xt_ctx* ctx, const xt_params* p, double* d_out, void* cuda_stream);
+
+/*
+ * Evaluations along the frozen grouping plan — the plan of the last successful xt_sum_logp / _host / _async evaluation
+ * (or of the one xt_chunk_logp ran).  The plan records hold only integers (groups, members, heads), so along them log P
+ * of every track is a smooth function of the parameters; finite differences of it give per-track scores and the
+ * observed information (tracking.param_uncertainty).  No plan kernel and no verification run: the replay kernel of the
+ * plan's own evaluation (fused, VAR, or the two-phase linear / log-domain kernel) runs once per parameter set, sized
+ * from the resident chunk summaries.  Nothing the objective keeps is changed: the next xt_sum_logp, xt_chunk_logp,
+ * xt_plan_dump, the verification state and the speculation counters return what they would have without these calls.
+ * Errors: XT_ERR_STATE without a resident plan (none yet, or discarded by xt_upload, xt_upload_aux,
+ * xt_set_stay_tables, xt_set_option or a failed evaluation); XT_ERR_ARG if a parameter set differs in structure (nS,
+ * nsub, d, n_loc, frame_len, flags) from the plan's evaluation; XT_ERR_UNSUPPORTED while "fp32_replay" is set (finite
+ * differences need FP64).
+ *
+ * xt_eval_frozen: n evaluations.  sums[k] = sum of log P over this context's tracks for ps[k], added in the fixed order
+ * xt_sum_logp uses (so at the plan's own parameters it has xt_sum_logp's bits).  track_logp (NULL = none):
+ * track_logp[k] = double[n_tracks], log P per track in upload order.
+ */
+int xt_eval_frozen(xt_ctx* ctx, int32_t n, const xt_params* ps, double* sums, double* const* track_logp);
+
+/*
+ * xt_score_outer: 2*n_dir evaluations along the same plan (1 <= n_dir <= XT_MAX_SCORE_DIRS).  With
+ * g[t][i] = (log P_t(p_plus[i]) - log P_t(p_minus[i])) * inv_2h[i]:  gsum[i] = sum_t g[t][i] and
+ * gram[i * n_dir + j] = sum_t g[t][i] g[t][j] (double[n_dir * n_dir], symmetric); sum_plus[i] / sum_minus[i] are the totals
+ * of the two evaluations.  The per-track vectors stay on the device: kernel k_score_gram forms g on the fly and
+ * accumulates per chunk in a fixed order; the chunk partials are added in chunk order.
+ */
+int xt_score_outer(xt_ctx* ctx, int32_t n_dir, const xt_params* p_plus, const xt_params* p_minus, const double* inv_2h,
+                   double* sum_plus, double* sum_minus, double* gsum, double* gram);
 
 /* Test seam = Proba_Cs (tracking.py:769-787): log P per track of chunk `chunk` after the last
  * xt_sum_logp call's parameters `p`.  out has nT[chunk] entries. */
@@ -303,6 +333,11 @@ int xt_multi_chunk_logp(xt_multi* m, int32_t chunk, const xt_params* p, double* 
 int xt_multi_set_option(xt_multi* m, const char* name, int value);
 /* share of device slot g (0 <= g < n_dev): CUDA ordinal, chunks and track-steps it owns */
 int xt_multi_device_load(xt_multi* m, int32_t g, int32_t* device, int32_t* n_chunks, int64_t* track_steps);
+/* xt_eval_frozen (sums only) / xt_score_outer over the devices: every device evaluates its chunks along its resident plan,
+ * the chunk partials are added in global chunk order (same bits for every n_dev, and as one context holding all chunks) */
+int xt_multi_eval_frozen(xt_multi* m, int32_t n, const xt_params* ps, double* sums);
+int xt_multi_score_outer(xt_multi* m, int32_t n_dir, const xt_params* p_plus, const xt_params* p_minus, const double* inv_2h,
+                         double* sum_plus, double* sum_minus, double* gsum, double* gram);
 /* counters of the last evaluation: sums over the devices; times and maxima are the max over the devices */
 int xt_multi_get_stats(xt_multi* m, xt_stats* out);
 
