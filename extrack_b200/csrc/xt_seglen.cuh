@@ -34,7 +34,7 @@ struct K4Args {
   int32_t Lmax;
   uint32_t* lattice;        // [gridDim.x][Lmax][cap]
   double* colmax;           // [gridDim.x][cap]: per column, max over the chunk's tracks of the final LP
-  double* hist;             // [n_chunks][Lmax][nS], accumulated with atomics
+  double* hist;             // [n_chunks][Lmax][nS], rows (L-1) x nS of every chunk written once by its CTA
   int32_t* flags;           // [0]: bit 0 = some chunk needed the > 600 rescale (informational); [1]: next position in corder
   const int32_t* corder;    // chunk ids, longest tracks first (CTAs take the next one when they are done)
   double leave_LL[XT_MAX_HEADS];  // log(pBL + (1-e) - pBL(1-e)) per head = newest + nS * previous
@@ -44,9 +44,17 @@ struct K4Args {
   int32_t dbg_chunk, dbg_nBf;
 };
 
+// two sets of (m[d], s2[KS], LP, LL), sort keys and indices, the chunk's histogram (FP64) and one track's fixed-point
+// histogram (int64), reduction slots, newest states
 __host__ __device__ inline size_t xt_seg_smem(int d, int KS, int cap, int n2, int Lmax, int nS) {
-  return (size_t)2 * cap * (d + KS + 2) * 8 + (size_t)n2 * 12 + (size_t)2 * cap + 16 + (size_t)Lmax * nS * 8 + 64;
+  return (size_t)2 * cap * (d + KS + 2) * 8 + (size_t)n2 * 12 + (size_t)2 * cap + 16 + (size_t)2 * Lmax * nS * 8 + 64;
 }
+
+// Fixed-point scale of a track's histogram: 2^(62 - bits(L)), so that L * scale < 2^62.  A track's weights sum to 1 and a
+// sequence adds its weight to one bin at most L times, so a bin stays below 2^62 plus the rounding of its additions
+// (< 2^15 * L of them): integer additions, exact and independent of their order.  The scale depends on the chunk's own L
+// only, so a chunk's histogram does not depend on what else is uploaded.
+__device__ __forceinline__ int xt_seg_fix_exp(int L) { return 62 - (32 - __clz(L)); }
 
 // "x comes before y" in the pruning order: descending key, equal keys by descending index
 __device__ __forceinline__ bool xt_seg_before(double kx, int ix, double ky, int iy) {
@@ -184,8 +192,9 @@ __global__ void __launch_bounds__(XT_SEG_THREADS, EPT == 4 ? 2 : 1) k4_seglen(co
   double* setB = setA + (size_t)cap * (D + KS + 2);
   double* keys = setB + (size_t)cap * (D + KS + 2);
   int* ord = reinterpret_cast<int*>(keys + n2);
-  double* shist = reinterpret_cast<double*>(ord + n2 + (n2 & 1));
-  double* sred = shist + (size_t)a.Lmax * nS;  // [8]
+  double* shist = reinterpret_cast<double*>(ord + n2 + (n2 & 1));                         // the chunk's rows
+  unsigned long long* sfix = reinterpret_cast<unsigned long long*>(shist + (size_t)a.Lmax * nS);  // one track's rows
+  double* sred = reinterpret_cast<double*>(sfix + (size_t)a.Lmax * nS);  // [8]
   uint8_t* stA = reinterpret_cast<uint8_t*>(sred + 8);
   uint8_t* stB = stA + cap;
   uint32_t* lat = a.lattice + (size_t)blockIdx.x * a.Lmax * cap;
@@ -207,8 +216,13 @@ __global__ void __launch_bounds__(XT_SEG_THREADS, EPT == 4 ? 2 : 1) k4_seglen(co
    const int ci = a.corder[pos];
    const XtChunk ck = a.chunks[ci];
    const int L = ck.L;
-   for (int i = tid; i < (L - 1) * nS; i += NT) shist[i] = 0.0;
+   // bin i of shist / sfix belongs to thread i % NT outside the run-length tally (reset, fold, store)
+   for (int i = tid; i < (L - 1) * nS; i += NT) {
+     shist[i] = 0.0;
+     sfix[i] = 0ull;
+   }
    for (int i = tid; i < cap; i += NT) colmax[i] = -INFINITY;
+   const double fix_scale = ldexp(1.0, xt_seg_fix_exp(L)), fix_inv = ldexp(1.0, -xt_seg_fix_exp(L));
    double cmax = -INFINITY;  // this thread's share of the chunk maximum of the final LP
    for (int pass = 0; pass < 2; ++pass) {
    for (int tk = 0; tk < ck.nT; ++tk) {
@@ -405,7 +419,23 @@ __global__ void __launch_bounds__(XT_SEG_THREADS, EPT == 4 ? 2 : 1) k4_seglen(co
     (void)mx;
     // ---- histories by walking the lattice back; run lengths (histograms.py:248-258 restated) ----
     for (int p = tid; p < nB; p += NT) {
-      const double w = keys[p] / tot;
+      const double w = keys[p] / tot;  // in [0, 1], or NaN when every weight of the track underflowed
+      // weight in fixed point: integer additions into the track's bins, so the tally does not depend on thread order
+      // (a NaN weight goes to the chunk's FP64 row directly: NaN in any order).  The 64-bit addition runs as two native
+      // 32-bit shared atomics, the low word's carry added to the high word (a 64-bit shared atomicAdd is a CAS loop).
+      const bool fin = isfinite(w);
+      const unsigned long long wq = fin ? (unsigned long long)__double2ll_rn(__dmul_rn(w, fix_scale)) : 0ull;
+      const unsigned wlo = (unsigned)wq, whi = (unsigned)(wq >> 32);
+      auto tally = [&](int bin) {
+        if (fin) {
+          unsigned* f = reinterpret_cast<unsigned*>(sfix + bin);  // little-endian: [0] low word, [1] high word
+          const unsigned old = atomicAdd(f, wlo);
+          const unsigned hi = whi + (old + wlo < old ? 1u : 0u);
+          if (hi) atomicAdd(f + 1, hi);
+        } else {
+          atomicAdd(&shist[bin], w);
+        }
+      };
       int idx = p;
       int cur = -1, run = 0, counted = 0, col = 0;
       int8_t* bs = (a.dbg_Bs && wk.chunk == a.dbg_chunk) ? a.dbg_Bs + ((size_t)wk.t0 * a.dbg_nBf + (size_t)p * (ck.isBL ? nS : 1)) * L
@@ -420,7 +450,7 @@ __global__ void __launch_bounds__(XT_SEG_THREADS, EPT == 4 ? 2 : 1) k4_seglen(co
           ++run;
         } else {
           if (cur >= 0) {
-            atomicAdd(&shist[(run - 1) * nS + cur], w);
+            tally((run - 1) * nS + cur);
             counted += run;
           }
           cur = st;
@@ -436,9 +466,15 @@ __global__ void __launch_bounds__(XT_SEG_THREADS, EPT == 4 ? 2 : 1) k4_seglen(co
       visit((int)(e0 >> 16));
       visit((int)(e0 & 0xFFFFu));
       const int last = L - counted;
-      if (last <= L - 1) atomicAdd(&shist[(last - 1) * nS + cur], w);
+      if (last <= L - 1) tally((last - 1) * nS + cur);
     }
     __syncthreads();
+    // fold the track's bins into the chunk's rows, track after track (the next track's tally starts after the
+    // barriers of its first step)
+    for (int i = tid; i < (L - 1) * nS; i += NT) {
+      shist[i] = __dadd_rn(shist[i], __dmul_rn((double)(long long)sfix[i], fix_inv));
+      sfix[i] = 0ull;
+    }
    }  // tracks of the chunk
    if (pass == 0) {  // did any final LP of the chunk exceed 600?  then once more with the column shifts
 #pragma unroll
@@ -458,7 +494,7 @@ __global__ void __launch_bounds__(XT_SEG_THREADS, EPT == 4 ? 2 : 1) k4_seglen(co
    }
    }  // passes
    double* gh = a.hist + (size_t)ci * a.Lmax * nS;
-   for (int i = tid; i < (L - 1) * nS; i += NT) gh[i] = shist[i];  // one CTA per chunk: plain stores, deterministic
+   for (int i = tid; i < (L - 1) * nS; i += NT) gh[i] = shist[i];  // one CTA per chunk: plain stores
    __syncthreads();
   }
 }

@@ -45,10 +45,25 @@ def _logdens_next(Cn, m, s2, l2):
     return np.sum(-0.5 * np.log(2 * np.pi * ns2) - (Cn - m) ** 2 / (2 * ns2), axis=2)
 
 
+def _min_rel_gap(key: np.ndarray) -> np.ndarray:
+    """Per row: the smallest non-zero relative gap between adjacent finite keys of the sorted row (inf if none)."""
+    s = np.sort(key, axis=1)
+    a, b = s[:, :-1], s[:, 1:]
+    with np.errstate(invalid="ignore"):
+        g = np.abs(b - a) / np.maximum(np.maximum(np.abs(a), np.abs(b)), 1e-300)
+    g = np.where(np.isfinite(a) & np.isfinite(b) & (g > 0), g, np.inf)
+    return g.min(axis=1) if g.shape[1] else np.full(len(key), np.inf)
+
+
 def segment_len_chunk(C: np.ndarray, model: Model, isBL: int, max_nb_states: int = 1000, min_l: int = 3,
-                      want_histories: bool = False):
+                      want_histories: bool = False, ties_ascending: bool = False, want_gaps: bool = False):
     """One chunk ``C[nT, L, d]`` (forward time).  Returns ``(LP[nT, nB], hist[L-1, nS])`` and, if
-    asked, the state histories ``[nT, nB, L]`` (column 0 = newest, like the reference's ``cur_Bs``)."""
+    asked, the state histories ``[nT, nB, L]`` (column 0 = newest, like the reference's ``cur_Bs``).
+
+    Test-only options: ``ties_ascending`` orders equal sort keys by *ascending* index (the reverse of
+    the documented rule), which shows whether a case has ties that change the result; ``want_gaps``
+    appends, per track, the smallest non-zero relative gap between adjacent sort keys over all pruning
+    steps (``inf`` without pruning) — where a last-bit difference of a library ``log`` could reorder keys."""
     if model.nb_substeps != 1:
         raise NotImplementedError("segment-length oracle: nb_substeps = 1 only")
     C = np.asarray(C, dtype=float)
@@ -71,6 +86,7 @@ def segment_len_chunk(C: np.ndarray, model: Model, isBL: int, max_nb_states: int
     s2 = np.repeat(l2 + tb.dd[None, :, None], nT, 0)
     state = np.repeat(newest[None], nT, 0)            # newest state per live sequence
     lattice = [(np.repeat((parent_state)[None], nT, 0), state.copy())]  # (oldest state as "parent", newest)
+    gaps = np.full(nT, np.inf)
     step = 2
     while step <= L - 1:
         nB = state.shape[1]
@@ -96,8 +112,12 @@ def segment_len_chunk(C: np.ndarray, model: Model, isBL: int, max_nb_states: int
         parent = np.repeat(par[None], nT, 0)
         if step < L - 1 and nB * nS > max_nb_states:
             key = LP + _logdens_next(C[:, None, step, :], m, s2, l2)
-            # descending key, ties by descending index
-            order = np.argsort(key, axis=1, kind="stable")[:, ::-1]
+            if ties_ascending:  # descending key, ties by ascending index
+                order = np.argsort(-key, axis=1, kind="stable")
+            else:  # descending key, ties by descending index
+                order = np.argsort(key, axis=1, kind="stable")[:, ::-1]
+            if want_gaps:
+                gaps = np.minimum(gaps, _min_rel_gap(key))
             k = max_nb_states
             top = order[:, :k]
             m = np.take_along_axis(m, top[:, :, None], 1)
@@ -158,9 +178,7 @@ def segment_len_chunk(C: np.ndarray, model: Model, isBL: int, max_nb_states: int
     last = L - counted                                    # the oldest run; a run of L (no transition) is not counted
     sel = last <= L - 1
     np.add.at(hist, (last[sel] - 1, cur[sel]), Pn[sel])
-    if want_histories:
-        return LP, hist, H
-    return LP, hist
+    return (LP, hist) + ((H,) if want_histories else ()) + ((gaps,) if want_gaps else ())
 
 
 def len_hist(sorted_tracks: Sequence[np.ndarray], model: Model, max_nb_states: int = 500) -> np.ndarray:

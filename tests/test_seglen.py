@@ -70,21 +70,20 @@ def test_gpu_P_segment_len_matches_reference_golden(path):
                                  dict(nS=3, L=15, d=2, mx=500, isBL=0, nT=23, min_l=5),
                                  dict(nS=2, L=25, d=3, mx=200, isBL=1, nT=50, min_l=3, le=(0.02, 0.025, 0.04))])
 def test_gpu_segment_len_vs_oracle_seeded(cfg):
-    """Default-sized pruning (max_nb_states 500: 1000 / 1500 live sequences per track) against the oracle."""
+    """Default-sized pruning (max_nb_states 500: 1000 / 1500 live sequences per track) against the oracle: histories per
+    track identical unless the oracle finds a near-tie of the sort keys there (test_seglen_edges.check_chunk)."""
     import sys
     sys.path.insert(0, GOLDEN)
     from helpers import random_walk_tracks
     from make_golden_seglen import model
+    from test_seglen_edges import check_chunk, oracle_chunk
     from extrack_b200 import histograms as xh
 
     m = model(cfg["nS"], cfg.get("le", (0.02,)))
     C = random_walk_tracks(cfg["nT"], cfg["L"], cfg["d"], np.random.default_rng(5), Ds=m.ds**2 / 0.04)
-    LP0, h0, H0 = so.segment_len_chunk(C, m, cfg["isBL"], cfg["mx"], cfg["min_l"], want_histories=True)
     LP, Bs, hist = xh.P_segment_len(C, np.asarray(m.loc_err)[None, None], m.ds, m.Fs, m.TrMat, min_l=cfg["min_l"], pBL=m.pBL,
                                     isBL=cfg["isBL"], cell_dims=[1.0], nb_substeps=1, max_nb_states=cfg["mx"])
-    np.testing.assert_allclose(LP, LP0, rtol=1e-9)
-    assert (Bs != H0).mean() < 1e-3   # a last-bit difference of a library log may swap two neighbours of the order
-    np.testing.assert_allclose(hist, h0, atol=1e-6)
+    assert check_chunk(LP, Bs, hist, oracle_chunk(C, m, cfg["isBL"], cfg["mx"], cfg["min_l"]), str(cfg)) <= 0.05 * cfg["nT"]
     # size-independent properties: every track contributes weight <= number of segments; rows beyond L-1 empty
     assert hist.shape == (cfg["L"] - 1, cfg["nS"]) and (hist >= 0).all()
 
