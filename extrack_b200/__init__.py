@@ -3,8 +3,8 @@
 Only the hot path of ``extrack.tracking`` is provided: ``param_fitting`` / ``cum_Proba_Cs`` /
 ``Proba_Cs`` / ``predict_Bs`` and the parameter builders (plus ``predict_transitions`` / ``transition_summary``: the
 per-step two-state posteriors of the same annotation, and ``predict_residuals``: its one-step-ahead predictive
-densities and PIT values, and ``predict_path`` / ``path_segments``: its most probable state paths and their dwell
-times), and ``param_uncertainty``: standard errors of fitted parameters from per-track scores along the frozen grouping
+densities and PIT values, ``predict_path`` / ``path_segments``: its most probable state paths and their dwell
+times, and ``sample_paths`` / ``sample_segments``: posterior draws of whole state paths and their dwell times), and ``param_uncertainty``: standard errors of fitted parameters from per-track scores along the frozen grouping
 plan, plus the data formats either side of it:
 ``readers.read_table`` (table -> length-bucketed ``all_tracks``) and ``simulate.sim_tracks``.  See DESIGN.md.
 """
@@ -24,6 +24,8 @@ from .tracking import (  # noqa: F401
     predict_path,
     predict_residuals,
     predict_transitions,
+    sample_paths,
+    sample_segments,
     transition_summary,
 )
 

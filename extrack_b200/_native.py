@@ -92,6 +92,7 @@ EXPORTS = (
     "xt_predict_pairs",
     "xt_predict_residuals",
     "xt_predict_path",
+    "xt_predict_samples",
     "xt_refine_positions",
     "xt_get_stats",
     "xt_seglen_hist",
@@ -154,6 +155,7 @@ def load_library() -> C.CDLL:
     lib.xt_predict_pairs.argtypes = [vp, P(XtParams), P(vp), P(vp)]
     lib.xt_predict_residuals.argtypes = [vp, P(XtParams), P(vp), P(vp), P(vp)]
     lib.xt_predict_path.argtypes = [vp, P(XtParams), P(vp), P(vp), P(vp)]
+    lib.xt_predict_samples.argtypes = [vp, P(XtParams), i32, C.c_uint64, P(i64), P(vp), P(vp), P(vp)]
     lib.xt_refine_positions.argtypes = [vp, P(XtParams), P(XtParams), P(vp), P(vp)]
     lib.xt_get_stats.argtypes = [vp, P(XtStats)]
     lib.xt_seglen_hist.argtypes = [vp, P(XtParams), P(dbl), P(dbl), i32, i32, vp, vp, P(i32)]
@@ -411,6 +413,23 @@ class Engine:
         arr = lambda xs: (C.c_void_p * len(xs))(*[o.ctypes.data for o in xs])
         self._check(self._lib.xt_predict_path(self._h, C.byref(p), arr(outs), arr(paths), arr(logps)))
         return outs, paths, logps
+
+    def predict_samples(self, p: XtParams, nS: int, n_samples: int, seed: int, row0: Optional[Sequence[int]] = None):
+        """``predict`` plus ``n_samples`` posterior draws of whole state paths per track: int8[n, n_samples, L] labels
+        and float64[n, n_samples] log route weights per uploaded segment (``xt_predict_samples``).  ``row0[s]``: the
+        caller's row of segment s's first track, the Philox counter of the draws (None: all 0)."""
+        outs = [np.empty((n, L, nS), dtype=np.float64) for (L, n) in self.segments]
+        smp = [np.empty((n, int(n_samples), L), dtype=np.int8) for (L, n) in self.segments]
+        logps = [np.empty((n, int(n_samples)), dtype=np.float64) for (L, n) in self.segments]
+        arr = lambda xs: (C.c_void_p * len(xs))(*[o.ctypes.data for o in xs])
+        r0 = None
+        if row0 is not None:
+            if len(row0) != len(self.segments):
+                raise ValueError("row0 needs one entry per uploaded segment")
+            r0 = (C.c_int64 * len(row0))(*[int(r) for r in row0])
+        self._check(self._lib.xt_predict_samples(self._h, C.byref(p), int(n_samples), C.c_uint64(int(seed)), r0, arr(outs),
+                                                 arr(smp), arr(logps)))
+        return outs, smp, logps
 
     def refine_positions(self, p_rev: XtParams, p_fwd: XtParams):
         """Refined positions [n, L, d] and their standard deviations [n, L] per uploaded segment (every segment

@@ -6,8 +6,8 @@
 
 // The own-plan annotation kernel of a model: scalar models with 2 or 3 states and the hot scratch in shared memory get
 // the instantiation with the number of states fixed at compile time (NSC), everything else the generic one.  `OUT`: the
-// instantiation that also writes the two-slice posteriors (K3Args::pairs), the residuals (K3Args::resid) or the MAP
-// paths (K3Args::path).
+// instantiation that also writes the two-slice posteriors (K3Args::pairs), the residuals (K3Args::resid), the MAP
+// paths (K3Args::path) or the posterior samples (K3Args::sample).
 using K3Kern = void (*)(const K3Args, const xt_params);
 struct K3Pick {
   K3Kern kern;
@@ -16,7 +16,8 @@ struct K3Pick {
 template <int D, int KS, bool VAR, int NSC, K3Out OUT>
 static K3Pick k3_one() {
   static unsigned long long smem_ok = 0;
-  return K3Pick{k3_predict<D, KS, VAR, false, false, NSC, OUT == K3_OUT_PAIRS, OUT == K3_OUT_RESID, OUT == K3_OUT_PATH>,
+  return K3Pick{k3_predict<D, KS, VAR, false, false, NSC, OUT == K3_OUT_PAIRS, OUT == K3_OUT_RESID, OUT == K3_OUT_PATH,
+                                OUT == K3_OUT_SAMPLE>,
                 &smem_ok};
 }
 template <int D, int KS, K3Out OUT>
@@ -33,6 +34,7 @@ static K3Pick k3_pick(const xt_params& p, int hot_smem, K3Out out) {
   k = out == K3_OUT_PAIRS   ? k3_pick_nsc<D_, KS_, K3_OUT_PAIRS>(var, nsc)       \
       : out == K3_OUT_RESID ? k3_pick_nsc<D_, KS_, K3_OUT_RESID>(var, nsc)       \
       : out == K3_OUT_PATH  ? k3_pick_nsc<D_, KS_, K3_OUT_PATH>(var, nsc)        \
+      : out == K3_OUT_SAMPLE ? k3_pick_nsc<D_, KS_, K3_OUT_SAMPLE>(var, nsc)     \
                             : k3_pick_nsc<D_, KS_, K3_OUT_PREDS>(var, nsc)
   XT_DISPATCH(p.d, p.n_loc, PICK_K3);
 #undef PICK_K3
@@ -71,7 +73,8 @@ cudaError_t xt_launch_k3_shared_plan(const K3SArgs& a, const xt_params& p, int g
 }
 template <int D, int KS, K3Out OUT>
 static cudaError_t launch_k3f(const K3Args& a, const xt_params& p, int grid, int nwarps, size_t smem, cudaStream_t stream) {
-  auto kern = k3_predict<D, KS, false, true, false, 0, OUT == K3_OUT_PAIRS, OUT == K3_OUT_RESID, OUT == K3_OUT_PATH>;
+  auto kern = k3_predict<D, KS, false, true, false, 0, OUT == K3_OUT_PAIRS, OUT == K3_OUT_RESID, OUT == K3_OUT_PATH,
+                                OUT == K3_OUT_SAMPLE>;
   static unsigned long long smem_ok = 0;
   cudaError_t e = xt_allow_smem(kern, smem, &smem_ok);
   if (e != cudaSuccess) return e;
@@ -85,6 +88,7 @@ cudaError_t xt_launch_k3_follow(const K3Args& a, const xt_params& p, int grid, i
   e = out == K3_OUT_PAIRS   ? launch_k3f<D_, KS_, K3_OUT_PAIRS>(a, p, grid, nwarps, smem, stream)        \
       : out == K3_OUT_RESID ? launch_k3f<D_, KS_, K3_OUT_RESID>(a, p, grid, nwarps, smem, stream)        \
       : out == K3_OUT_PATH  ? launch_k3f<D_, KS_, K3_OUT_PATH>(a, p, grid, nwarps, smem, stream)         \
+      : out == K3_OUT_SAMPLE ? launch_k3f<D_, KS_, K3_OUT_SAMPLE>(a, p, grid, nwarps, smem, stream)      \
                             : launch_k3f<D_, KS_, K3_OUT_PREDS>(a, p, grid, nwarps, smem, stream)
   XT_DISPATCH(p.d, p.n_loc, CALL_K3F);
 #undef CALL_K3F

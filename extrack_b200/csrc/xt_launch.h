@@ -13,7 +13,7 @@ struct K3SArgs;
 struct KRArgs;
 struct K4Args;
 // what a state-annotation launch writes next to the posteriors (selects the k3_predict instantiation)
-enum K3Out { K3_OUT_PREDS = 0, K3_OUT_PAIRS = 1, K3_OUT_RESID = 2, K3_OUT_PATH = 3 };
+enum K3Out { K3_OUT_PREDS = 0, K3_OUT_PAIRS = 1, K3_OUT_RESID = 2, K3_OUT_PATH = 3, K3_OUT_SAMPLE = 4 };
 
 #define XT_DISPATCH(D_, KS_, CALL)                                   \
   do {                                                               \
@@ -61,7 +61,7 @@ cudaError_t xt_launch_k2_f32(int d, int ks, const K2FArgs& a, const K2Tab& tab, 
 cudaError_t xt_launch_k2_old(const K2Args& a, const xt_params& p, const K2Lin& lin, size_t smem, bool use_smem, int grid,
                              int wpc, cudaStream_t stream);
 // state annotation (xt_predict.cuh); `out`: the instantiation that also writes the two-slice posteriors (a.pairs), the
-// residuals (a.resid) or the MAP paths (a.path)
+// residuals (a.resid), the MAP paths (a.path) or the posterior samples (a.sample)
 cudaError_t xt_launch_k3(const K3Args& a, const xt_params& p, int grid, int nwarps, size_t smem, cudaStream_t stream, K3Out out);
 int xt_k3_regs(const xt_params& p, int hot_smem, K3Out out);  // registers per thread of the kernel xt_launch_k3 would launch
 // ... with plans shared by the nb_max tracks of a chunk (xt_predict_shared.cuh): the plans, then the annotation along them

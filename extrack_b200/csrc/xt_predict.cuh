@@ -36,15 +36,35 @@
 //     path_logp = V* - logsumexp(final LP) = log(weight of the heaviest route)
 // by telescoping.  Without fusion V = LP, so the path is the exact argmax over the state sequences
 // (oracle/path_oracle.py).
+// With SAMPLE the kernel also draws whole routes of that lattice with probability equal to their weight (forward
+// filtering, backward sampling): the final sequence c with the final weights aC, then for s = L-1 down to 3 the label of
+// c at localisation s and one member of its parent group c / K (a group of the fusion at step s - 1) with the recorded
+// normalised weights rw, in member order; at s = 2 the parent is the initial sequence h0 + nS*h1 (labels h0 at 1, h1
+// at 0).  Every choice among n >= 2 candidates takes the first k with u*S < cum_k (cum: the running FP64 sums of the
+// candidates' weights in order, S = cum_n-1; if rounding leaves none, the last candidate of positive weight), with
+//     u = Philox4x32-10(counter {row, L, draw, level}, key {seed lo, seed hi}) (xt_philox.cuh)
+// row = the track's row in the caller's bucket, level = L - 1 for the final choice and s - 1 for a member choice, so a
+// draw depends on nothing but (seed, L, row, draw) and the track.  sample_logp = log aC[final] + sum of log rw along the
+// route (oracle/sample_oracle.py).
 #pragma once
 #include <math_constants.h>
 #include "xt_common.cuh"
+#include "xt_philox.cuh"
 #include "xt_plan.cuh"
 
 #define XT_K3_WARPS 8
 #ifndef XT_K3_MIN_CTAS
 #define XT_K3_MIN_CTAS 2  // resident CTAs of 8 warps the register allocation leaves room for (2: 128 registers)
 #endif
+
+// SAMPLE instantiation: what the draws need besides K3Args (a device struct, so that K3Args keeps its size)
+struct K3SampleOut {
+  int8_t* labels;        // int8[sum over tracks of L][n]: a track's draws from (loc_off + t L) n on, draw d at + d L
+  double* logp;          // double[n_tracks][n]: (trk_off + t) n + d
+  const int64_t* row0;   // [uploaded segments]: the caller's row of the segment's first track (Philox counter word 0)
+  uint64_t seed;         // Philox key
+  int32_t n;             // draws per track
+};
 
 struct K3Args {
   const XtChunk* chunks;
@@ -82,6 +102,8 @@ struct K3Args {
     // pointers to int8_t[sum over tracks of L] in forward time (a track's labels at loc_off + t L) and double[n_tracks]
     // (a track's entry at trk_off + t)
     void* const* path;
+    // SAMPLE instantiation (sample_paths, never REFINE, PAIRS, RESID nor PATH): its outputs, stream and rows
+    const struct K3SampleOut* sample;
   };
   const int64_t* dump_off;
   int32_t* ent_n;        // [n_chunks][maxL]: sequences per entry (written by the chunk's first track)
@@ -118,7 +140,27 @@ struct K3PathPtrs {
   double* vC;        // ... of the children [cap]
   uint16_t* recArg;  // [maxL][cap / nS + 1]: argmax member of every group of every fused step
 };
-template <bool PATH = false>
+// SAMPLE instantiation: its own cold regions after those of the other modes' layout `l` (own-plan mode: the member lists
+// of every fused step, which the shared plan of FOLLOW already holds), and the cold total that includes them
+struct K3SampleLayout {
+  size_t order, goff, cum, cold_total;  // uint16[maxL][cap], uint16[maxL][cap + 1], double[cap]
+};
+__host__ __device__ inline K3SampleLayout k3_sample_layout(const K3Layout& l, int cap, int maxL) {
+  K3SampleLayout q;
+  size_t o = l.cold_total;
+  q.order = o;  o += ((size_t)maxL * cap + 3) / 4;
+  q.goff = o;   o += ((size_t)maxL * (cap + 1) + 3) / 4;
+  q.cum = o;    o += cap;
+  q.cold_total = o;
+  return q;
+}
+// The SAMPLE arrays of one warp (cold part at `cold`)
+struct K3SamplePtrs {
+  uint16_t* order;  // [maxL][cap]: members of the groups of every fused step, group by group in member order
+  uint16_t* goff;   // [maxL][cap + 1]: first member of every group in `order` (+ one past the end)
+  double* cum;      // [cap]: running sums of the final weights
+};
+template <bool PATH = false, bool SAMPLE = false>
 __host__ __device__ inline K3Layout k3_layout(int cap, int CO, int fl, int nS, int maxL) {
   K3Layout l;
   size_t o = 0;
@@ -148,11 +190,16 @@ __host__ __device__ inline K3Layout k3_layout(int cap, int CO, int fl, int nS, i
     l.hot_total = q.hot_total;
     l.cold_total = q.cold_total;
   }
+  if constexpr (SAMPLE) l.cold_total = k3_sample_layout(l, cap, maxL).cold_total;
   return l;
 }
 static __device__ __forceinline__ K3PathPtrs k3_path_ptrs(double* base, double* cold, int cap, int CO, int fl, int nS, int maxL) {
   const K3PathLayout q = k3_path_layout(k3_layout(cap, CO, fl, nS, maxL), cap, nS, maxL);
   return K3PathPtrs{base + q.vP, base + q.vC, (uint16_t*)(cold + q.recArg)};
+}
+static __device__ __forceinline__ K3SamplePtrs k3_sample_ptrs(double* cold, int cap, int CO, int fl, int nS, int maxL) {
+  const K3SampleLayout q = k3_sample_layout(k3_layout(cap, CO, fl, nS, maxL), cap, maxL);
+  return K3SamplePtrs{(uint16_t*)(cold + q.order), (uint16_t*)(cold + q.goff), cold + q.cum};
 }
 
 // The annotation kernel is sensitive to instruction fetch (ncu: 32 % of the stall samples were "no instruction" with
@@ -294,13 +341,14 @@ static __device__ __forceinline__ void k3_emit_resid(double* lp, double* pit, co
 }
 
 template <int D, int KS, bool VAR = false, bool FOLLOW = false, bool REFINE = false, int NSC = 0, bool PAIRS = false,
-          bool RESID = false, bool PATH = false>
+          bool RESID = false, bool PATH = false, bool SAMPLE = false>
 __global__ void __launch_bounds__(32 * XT_K3_WARPS, XT_K3_MIN_CTAS) k3_predict(const K3Args a, const __grid_constant__ xt_params P) {
   static_assert(!(VAR && FOLLOW), "shared plans are built for scalar LocErr / dt models");
   static_assert(!REFINE || FOLLOW, "the refinement recursion follows the bucket's shared plan");
   static_assert(!(REFINE && PAIRS), "the refinement stores no posteriors");
   static_assert(!(REFINE && RESID) && !(PAIRS && RESID), "the residuals share the output pointer of the other modes");
   static_assert(!(PATH && (REFINE || PAIRS || RESID)), "the MAP paths share the output pointer of the other modes");
+  static_assert(!(SAMPLE && (REFINE || PAIRS || RESID || PATH)), "the samples share the output pointer of the other modes");
   // NSC > 0: the number of states is the compile-time constant NSC and the hot scratch is known to be in shared memory
   // (32-bit shared-memory addressing, shifts / multiply-shifts instead of integer divisions); NSC == 0: both at run time
   constexpr bool HOT = NSC > 0;
@@ -320,7 +368,7 @@ __global__ void __launch_bounds__(32 * XT_K3_WARPS, XT_K3_MIN_CTAS) k3_predict(c
   };
 
   // ---- per-warp scratch carve-up ----
-  const K3Layout lay = k3_layout<PATH>(cap, CO, fl, nS, a.maxL);
+  const K3Layout lay = k3_layout<PATH, SAMPLE>(cap, CO, fl, nS, a.maxL);
   double* cold = a.scratch + (size_t)(blockIdx.x * nwarps + warp) * a.warp_scratch;
   double* base;
   if constexpr (HOT) base = k3_smem + warp * (int)lay.hot_total;
@@ -342,6 +390,8 @@ __global__ void __launch_bounds__(32 * XT_K3_WARPS, XT_K3_MIN_CTAS) k3_predict(c
   // PATH: its arrays (K3PathPtrs) are fetched inside the PATH-only blocks, so that the other instantiations compile to
   // exactly the code they had without this mode
 #define K3_PATH_PTRS const K3PathPtrs pa = k3_path_ptrs(base, cold, cap, CO, fl, nS, a.maxL)
+  // SAMPLE: likewise (K3SamplePtrs)
+#define K3_SAMPLE_PTRS const K3SamplePtrs sp = k3_sample_ptrs(cold, cap, CO, fl, nS, a.maxL)
 
   const int capP = cap / nS + 1;  // parent / group slots
 #define BP(slot, comp) bufP[(comp) * capP + (slot)]
@@ -667,6 +717,14 @@ __global__ void __launch_bounds__(32 * XT_K3_WARPS, XT_K3_MIN_CTAS) k3_predict(c
         __syncwarp();
         if (errc) break;
 
+        if constexpr (SAMPLE && !FOLLOW) {  // this step's member lists, for the draws
+          K3_SAMPLE_PTRS;
+          uint16_t* so = sp.order + (size_t)step * cap;
+          uint16_t* sg = sp.goff + (size_t)step * (cap + 1);
+          for (int g = lane; g <= nG; g += 32) sg[g] = (uint16_t)goff[g];
+          for (int c = lane; c < nC; c += 32) so[c] = (uint16_t)order[c];
+        }
+
         // ---- merge, lane = group (tracking.py:723-741); record normalised weights ----
         if (lane == 0) recN[step] = nC;
         const int rows_out = rows_cmp;  // window rows kept (older rows never influence a decision)
@@ -928,6 +986,84 @@ __global__ void __launch_bounds__(32 * XT_K3_WARPS, XT_K3_MIN_CTAS) k3_predict(c
           ((double*)a.path[1])[(size_t)ck.trk_off + t] = pbest - (log(ssum) + vmax);
         }
       }
+      if constexpr (SAMPLE) {
+        // posterior draws of whole routes, lane = draw (the backward sweep below overwrites aC)
+        K3_SAMPLE_PTRS;
+        const K3SampleOut so = *a.sample;
+        if (lane == 0) {
+          double acc = 0.0;
+          #pragma unroll 1
+          for (int c = 0; c < nP; ++c) {
+            acc = __dadd_rn(acc, aC[c]);
+            sp.cum[c] = acc;
+          }
+        }
+        __syncwarp();
+        const uint32_t row = (uint32_t)(so.row0[ck.seg] + ck.seg_t0 + t);
+        const int32_t* splan = FOLLOW ? a.splan + (size_t)wk.chunk * a.splan_stride + 2 * a.maxL : nullptr;
+        #pragma unroll 1
+        for (int dr = lane; dr < so.n; dr += 32) {
+          auto u01 = [&](int level) { return xt_philox_u01(row, (uint32_t)L, (uint32_t)dr, (uint32_t)level, so.seed); };
+          // the final sequence: the first c with u S < cum[c] (binary search: cum is non-decreasing)
+          int c = 0;
+          if (nP > 1) {
+            const double x = __dmul_rn(u01(L - 1), sp.cum[nP - 1]);
+            int lo = 0, hi = nP;
+            #pragma unroll 1
+            while (lo < hi) {
+              const int mid = (lo + hi) >> 1;
+              if (x < sp.cum[mid]) hi = mid;
+              else lo = mid + 1;
+            }
+            c = lo;
+            if (c == nP) {
+              c = nP - 1;
+              while (c > 0 && !(aC[c] > 0.0)) --c;
+            }
+          }
+          double lp = log(aC[c]);
+          int8_t* lab = so.labels + ((size_t)ck.loc_off + (size_t)t * L) * so.n + (size_t)dr * L;
+          #pragma unroll 1
+          for (int s = L - 1; s >= 3; --s) {
+            lab[s] = (int8_t)label(c);
+            const int p = c / K, level = s - 1;
+            // members of group p of the fusion at step `level`: its shared-plan entries (FOLLOW) or the own records
+            const int32_t* pl = FOLLOW ? splan + (size_t)level * (2 * cap + 1) : nullptr;
+            const uint16_t* ord = sp.order + (size_t)level * cap;
+            const int o = FOLLOW ? pl[p] : (int)sp.goff[(size_t)level * (cap + 1) + p];
+            const int n = (FOLLOW ? pl[p + 1] : (int)sp.goff[(size_t)level * (cap + 1) + p + 1]) - o;
+            auto member = [&](int k) { return FOLLOW ? (int)pl[cap + 1 + o + k] : (int)ord[o + k]; };
+            const double* rw = recW + (size_t)level * cap;
+            int pick = member(0);
+            if (n > 1) {
+              double S = 0.0;
+              #pragma unroll 1
+              for (int k = 0; k < n; ++k) S = __dadd_rn(S, rw[member(k)]);
+              const double x = __dmul_rn(u01(level), S);
+              double acc = 0.0;
+              int k = 0, last_pos = 0;
+              #pragma unroll 1
+              for (; k < n; ++k) {
+                const double w = rw[member(k)];
+                if (w > 0.0) last_pos = k;
+                acc = __dadd_rn(acc, w);
+                if (x < acc) break;
+              }
+              pick = member(k < n ? k : last_pos);
+            }
+            c = pick;
+            lp += log(rw[c]);
+          }
+          if (L >= 3) {
+            lab[2] = (int8_t)label(c);
+            c /= K;
+          }
+          lab[1] = (int8_t)(c % nS);  // initial sequence c = h0 + nS*h1: row 1 = h0, row 0 = h1
+          lab[0] = (int8_t)(c / nS);
+          so.logp[((size_t)ck.trk_off + t) * so.n + dr] = lp;
+        }
+        __syncwarp();
+      }
 
       // ---- backward sweep over the recorded lattice (deterministic warp reductions) ----
       // aC holds the posterior of the sequences *after* the expansion of `step`.
@@ -1015,4 +1151,5 @@ __global__ void __launch_bounds__(32 * XT_K3_WARPS, XT_K3_MIN_CTAS) k3_predict(c
 #undef DDX
 #undef LROW
 #undef K3_PATH_PTRS
+#undef K3_SAMPLE_PTRS
 }

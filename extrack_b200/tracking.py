@@ -804,6 +804,74 @@ def predict_path(all_tracks, dt, params, cell_dims=[1], nb_states=4, frame_len=5
                      gather, "path")
 
 
+def sample_paths(all_tracks, dt, params, cell_dims=[1], nb_states=4, frame_len=5, max_nb_states=200, threshold=0.1,
+                 workers=1, input_LocErr=None, verbose=0, nb_max=1, gather=True, n_samples=100, seed=0):
+    """``predict_Bs`` plus ``n_samples`` posterior draws of the whole state path of every track: ``(preds, samples,
+    sample_logp)``, three ``{str(L): array}`` dictionaries.  ``preds[k]`` is ``predict_Bs``'s float64[n, L,
+    nb_states]; ``samples[k]`` is int8[n, n_samples, L], one state label per localisation and draw (forward time);
+    ``sample_logp[k]`` is float64[n, n_samples].
+
+    The draws run on the lattice of ``predict_path`` (forward filtering, backward sampling): a draw picks a route with
+    probability equal to its weight, from the end backwards (the final sequence with the final softmax weights, then at
+    every fusion one member of the parent group with its normalised merge weight).  ``sample_logp`` is the log of the
+    drawn route's weight, so it never exceeds ``predict_path``'s ``path_logp``.  Over the draws, the frequency of label
+    i at localisation k converges to ``preds[t, k, i]`` and that of consecutive labels to ``predict_transitions``'
+    pairs; without fusion (tracks no longer than ``frame_len``) every draw is an exact sample of the posterior
+    P(s_0..s_L-1 | track).  The mean over draws of any path statistic (dwell times, switches per track, time to the
+    first switch) is its posterior expectation and the spread over draws its credible interval; ``sample_segments``
+    gives the dwell-time histogram of every draw.  Labels are those of ``preds`` (with the reference's int8 label wrap).
+
+    The draws are reproducible: they depend only on ``seed``, the bucket length, the track's row in its bucket and the
+    draw index, so draw d is the same whatever ``n_samples`` (>= d + 1), ``torch.distributed`` sharding or launch
+    shape.  ``n_samples`` must be an int in [1, 65535] and ``seed`` an int in [0, 2^64).  Other arguments, validation,
+    ``nb_max`` rules and errors, sharding and ``gather`` are those of ``predict_Bs`` (the samples and their log weights
+    take one more all-gather per bucket each).
+    """
+    _int = lambda x: isinstance(x, (int, np.integer)) and not isinstance(x, (bool, np.bool_))
+    if not _int(n_samples) or not 1 <= int(n_samples) <= 65535:
+        raise ValueError("n_samples must be an int in [1, 65535]")
+    if not _int(seed) or not 0 <= int(seed) < 2**64:
+        raise ValueError("seed must be an int in [0, 2^64)")
+    return _annotate(all_tracks, dt, params, cell_dims, nb_states, frame_len, max_nb_states, threshold, input_LocErr, nb_max,
+                     gather, "samples", int(n_samples), int(seed))
+
+
+def _segments(a):
+    """Maximal runs of equal labels in the rows of a [n, L] (int64): (row, length, state, censored) of every run, in
+    row-major order.  A run is censored when it touches the first or the last localisation of its row."""
+    n, L = a.shape
+    change = a[:, 1:] != a[:, :-1]  # [n, L - 1]: a segment ends at localisation k and the next starts at k + 1
+    t_e, k_e = np.nonzero(np.concatenate([change, np.ones((n, 1), dtype=bool)], axis=1))
+    _, k_s = np.nonzero(np.concatenate([np.ones((n, 1), dtype=bool), change], axis=1))
+    # (row-major order: the i-th start and the i-th end belong to the same segment)
+    return t_e, k_e - k_s + 1, a[t_e, k_e], (k_s == 0) | (k_e == L - 1)
+
+
+def sample_segments(samples, nb_states):
+    """Dwell-time histograms of ``sample_paths``' draws (host only): ``(interior, censored)``, two int64 arrays
+    [n_samples, L_max, nb_states].  Slice d is ``path_segments`` of draw d over all tracks: row ``n - 1`` counts the
+    segments of n localisations by state, ``interior`` those with both ends observed inside the track, ``censored``
+    those touching its first or last localisation.  The mean over the first axis is the posterior expectation of the
+    histogram and its quantiles over that axis are credible bands."""
+    items = [np.asarray(a) for a in (samples.values() if isinstance(samples, dict) else samples)]
+    items = [a for a in items if a.ndim == 3]
+    L_max = max((a.shape[2] for a in items), default=0)
+    S = items[0].shape[1] if items else 0
+    if any(a.shape[1] != S for a in items):
+        raise ValueError("every bucket must hold the same number of draws")
+    interior = np.zeros((S, L_max, nb_states), dtype=np.int64)
+    censored = np.zeros((S, L_max, nb_states), dtype=np.int64)
+    for a in items:
+        if a.size == 0:
+            continue
+        n, _, L = a.shape
+        row, length, state, cens = _segments(a.astype(np.int64).reshape(n * S, L))
+        draw = row % S
+        np.add.at(interior, (draw[~cens], length[~cens] - 1, state[~cens]), 1)
+        np.add.at(censored, (draw[cens], length[cens] - 1, state[cens]), 1)
+    return interior, censored
+
+
 def path_segments(paths, nb_states):
     """Run lengths of the MAP segments of ``predict_path``'s paths (host only): ``(interior, censored)``, two int64
     arrays [L_max, nb_states] (L_max: the longest bucket's length).  Row ``n - 1`` counts the segments of n
@@ -818,14 +886,7 @@ def path_segments(paths, nb_states):
     for a in items:
         if a.size == 0:
             continue
-        a = a.astype(np.int64)
-        n, L = a.shape
-        change = a[:, 1:] != a[:, :-1]  # [n, L - 1]: a segment ends at localisation k and the next starts at k + 1
-        t_e, k_e = np.nonzero(np.concatenate([change, np.ones((n, 1), dtype=bool)], axis=1))
-        _, k_s = np.nonzero(np.concatenate([np.ones((n, 1), dtype=bool), change], axis=1))
-        # (row-major order: the i-th start and the i-th end belong to the same segment)
-        length, state = k_e - k_s + 1, a[t_e, k_e]
-        cens = (k_s == 0) | (k_e == L - 1)
+        _, length, state, cens = _segments(a.astype(np.int64))
         np.add.at(interior, (length[~cens] - 1, state[~cens]), 1)
         np.add.at(censored, (length[cens] - 1, state[cens]), 1)
     return interior, censored
@@ -855,9 +916,10 @@ def transition_summary(preds, pairs):
 
 
 def _annotate(all_tracks, dt, params, cell_dims, nb_states, frame_len, max_nb_states, threshold, input_LocErr, nb_max, gather,
-              kind):
-    """Body of predict_Bs ("preds"), predict_transitions ("pairs"), predict_residuals ("resid") and predict_path
-    ("path"): the posteriors and the arrays of that output kind, each as a {str(L): array} dictionary."""
+              kind, n_samples=0, seed=0):
+    """Body of predict_Bs ("preds"), predict_transitions ("pairs"), predict_residuals ("resid"), predict_path
+    ("path") and sample_paths ("samples", with n_samples and seed): the posteriors and the arrays of that output kind,
+    each as a {str(L): array} dictionary."""
     sorted_tracks, l_list = _sorted_buckets(all_tracks)
     keys = [k for k in l_list if len(all_tracks[k]) > 0]
     sorted_LocErrs = [np.asarray(input_LocErr[k], dtype=np.float64) for k in keys] if input_LocErr is not None else None
@@ -881,9 +943,10 @@ def _annotate(all_tracks, dt, params, cell_dims, nb_states, frame_len, max_nb_st
         "pairs": [lambda L: (L - 1, nb_states, nb_states)],
         "resid": [lambda L: (L,), lambda L: (L, d)],
         "path": [lambda L: (L,), lambda L: ()],
+        "samples": [lambda L: (n_samples, L), lambda L: (n_samples,)],
     }[kind]
-    # the paths are int8 labels (gathered as float64, exact for labels < 2^53, and cast back)
-    dtypes = [np.int8 if (kind == "path" and i == 1) else np.float64 for i in range(len(row_shapes))]
+    # the paths and samples are int8 labels (gathered as float64, exact for labels < 2^53, and cast back)
+    dtypes = [np.int8 if (kind in ("path", "samples") and i == 1) else np.float64 for i in range(len(row_shapes))]
     outs = [{l: np.empty((0,) + rs(int(l)), dtype=dt_) for l in l_list} for rs, dt_ in zip(row_shapes, dtypes)]
     if not sorted_tracks:
         return tuple(outs)
@@ -930,6 +993,9 @@ def _annotate(all_tracks, dt, params, cell_dims, nb_states, frame_len, max_nb_st
                 res = eng.predict_residuals(p, nb_states)
             elif kind == "path":
                 res = eng.predict_path(p, nb_states)
+            elif kind == "samples":
+                # the draws' Philox counter is the track's row in its whole bucket, not in this rank's slice
+                res = eng.predict_samples(p, nb_states, n_samples, seed, [cuts[b][0] for b in mine])
             else:
                 res = (eng.predict(p, nb_states),)
             for lo, arrs in zip(local, res):

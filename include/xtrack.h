@@ -243,6 +243,26 @@ int xt_predict_residuals(xt_ctx* ctx, const xt_params* p, double* const* out, do
 int xt_predict_path(xt_ctx* ctx, const xt_params* p, double* const* out, int8_t* const* path, double* const* path_logp);
 
 /*
+ * State annotation with posterior samples of whole state paths (forward filtering, backward sampling on the lattice of
+ * xt_predict_path): xt_predict (same options, plans and errors, same out[s]) that also fills samples[s] with
+ * int8_t[n[s]][n_samples][L[s]] and sample_logp[s] with double[n[s]][n_samples].  Draw d of track t picks a route with
+ * probability equal to its weight, from the end backwards: the final sequence with the final softmax weights, then at
+ * every fusion one member of the parent group with the normalised merge weights, in member order.
+ *   samples[s][t][d][k]   = the state label at localisation k of the drawn route (labels of out[s], int8 wrap included)
+ *   sample_logp[s][t][d]  = log of the drawn route's weight (<= the path_logp of xt_predict_path)
+ * The frequency of label i at localisation k over the draws converges to out[s][t][k][i]; without fusion every draw is an
+ * exact sample of P(s_0..s_L-1 | track).  Each choice among n >= 2 candidates takes the first k with u*S < cum_k (cum:
+ * running FP64 sums of the weights in order, S its last; none after rounding: the last candidate of positive weight),
+ * with u = ((x0 << 32 | x1) >> 11) * 2^-53 from Philox4x32-10, key {seed & 0xffffffff, seed >> 32}, counter
+ * {row, L, d, level}: row = row0[s] + the track's index in segment s (row0 NULL: all 0), level = L - 1 for the final
+ * choice and the fusion step (2 .. L - 2) for a member choice.  Draws therefore depend only on (seed, L, row, d) and the
+ * track: not on the launch, the chunking, n_samples or which other tracks are uploaded.
+ * XT_ERR_ARG: n_samples outside 1..65535, or a null out / samples / sample_logp.
+ */
+int xt_predict_samples(xt_ctx* ctx, const xt_params* p, int32_t n_samples, uint64_t seed, const int64_t* row0,
+                       double* const* out, int8_t* const* samples, double* const* sample_logp);
+
+/*
  * Position refinement — replaces extrack/refined_localization.py:207-338 (get_pos_PDF + the weighted means of
  * position_refinement) for the uploaded tracks.  Upload every length bucket as ONE chunk (chunk_size >= its track
  * count): the reference hands whole buckets to get_LC_Km_Ks (:48-204), whose grouping plan comes from the bucket's first
